@@ -8,10 +8,12 @@ Metric: impressions/s (whole job).  See DESIGN.md "Measurement" for every defini
 
   python bench.py --gpus N --steps K --warmup W            our arm (CUDA, sm_100a)
   python bench.py --impl reference ...                      the reference's algorithm on host cores
+  python bench.py ... --dump-outputs DIR                    also write the last timed step's outputs as DIR/*.npy
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -21,6 +23,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 import numpy as np
 import torch
@@ -72,7 +75,39 @@ def _parse_args():
                          "ranks by parallel.shard_impressions (balanced by sum(H + C))")
     ap.add_argument("--parity-impressions", type=int, default=12, help="impressions of the sampled fp64-oracle check (0 = skip)")
     ap.add_argument("--ref-cuda-batches", type=int, default=6, help="mini-batches of the reference-algorithm-on-CUDA leg (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0) as DIR/<name>.npy: scores [pairs] fp32, "
+                         "per_impression_metrics [impressions, 4] and metric_sums [5] fp64; at most 64 MB in all.  "
+                         "--impl reference: logits [batch, 1] fp32 of the last timed mini-batch")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Writes each array as <path>/<name>.npy.  If they hold more than DUMP_BYTES, every array larger than 1 MB keeps a
+    fixed, seeded sample of its rows (sorted) and <name>_rows.npy records which rows, so that two runs with the same
+    arguments write the same elements.  A <name>_rows.npy left in DIR by an earlier, sampled run is removed when <name>
+    is written whole."""
+    os.makedirs(path, exist_ok=True)
+    big = [k for k, a in arrays.items() if a.nbytes > 1 << 20]
+    room = DUMP_BYTES - sum(a.nbytes for k, a in arrays.items() if k not in big) - 2 * len(arrays) * 1024   # .npy headers
+    out = dict(arrays)
+    if sum(arrays[k].nbytes for k in big) > room:
+        frac = room / sum(arrays[k].nbytes + 8 * len(arrays[k]) for k in big)
+        for k in big:
+            rows = np.sort(np.random.default_rng(0).choice(len(arrays[k]), size=int(len(arrays[k]) * frac), replace=False))
+            out[k], out[k + "_rows"] = arrays[k][rows], rows.astype(np.float64)
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+    for k in arrays:
+        stale = os.path.join(path, k + "_rows.npy")
+        if k + "_rows" not in out and os.path.exists(stale):
+            os.remove(stale)
 
 
 def algorithmic_bytes(imp):
@@ -92,6 +127,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(index), "--query-gpu=" + self.Q,
                                           "--format=csv,noheader,nounits", "-lms", "200"],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)     # the sampler never outlives the benchmark, even one that fails
             self.t = threading.Thread(target=self._read, daemon=True)
             self.t.start()
         except OSError:
@@ -129,24 +165,28 @@ def make_setup(args, rank, need_news_text=True, world=1):
 
 def cpu_baseline(args, cfg, news, imp, model_sd, steps=None, warmup=0):
     """The reference's algorithm (oracle port: per-pair batches, 51 news encodes per pair,
-    util.py:88-112) on the host cores, on a bounded sample of the same workload."""
+    util.py:88-112) on the host cores, on a bounded sample of the same workload: the first full mini-batches of the
+    impression set, --cpu-pairs pairs of them, or exactly warmup + steps batches when steps is given."""
     from oracle import lime_oracle as O
     from lime_cikm25_b200 import synth
     cores = os.cpu_count() or 1
     torch.set_num_threads(cores)
     bs = args.batch_size
     batches = []
-    for b in synth.impressions_to_pair_batches(news, imp.slice(0, min(imp.num_impressions, 64)), bs):
+    for b in synth.impressions_to_pair_batches(news, imp, bs):      # a generator: only the batches taken are built
         if len(b[0]) == bs:
             batches.append(b)
         if len(batches) * bs >= (args.cpu_pairs if steps is None else bs * (steps + warmup)):
             break
+    if steps is not None and len(batches) < steps + warmup:
+        raise SystemExit("bench.py: the impression set holds %d full mini-batches of %d pairs, fewer than --warmup + --steps = %d"
+                         % (len(batches), bs, steps + warmup))
     cbar = float(np.mean(np.diff(imp.cand_off)))
     times = []
     with torch.no_grad():
         for i, b in enumerate(batches):
             t0 = time.perf_counter()
-            O.model_forward(model_sd, b, cfg)
+            logits = O.model_forward(model_sd, b, cfg)
             times.append(time.perf_counter() - t0)
     timed = times[warmup:] if len(times) > warmup else times
     pairs_s = bs * len(timed) / sum(timed)
@@ -154,7 +194,7 @@ def cpu_baseline(args, cfg, news, imp, model_sd, steps=None, warmup=0):
             "sample": "%d mini-batches of %d (user,candidate) pairs, each pair re-encoding %d news as "
                       "util.py:88-112 does; %.1f pairs/s; converted with mean %.1f candidates/impression"
                       % (len(timed), bs, H + 1, pairs_s, cbar),
-            "pairs_per_sec": pairs_s, "ms_per_step": 1e3 * sum(timed) / len(timed)}
+            "pairs_per_sec": pairs_s, "ms_per_step": 1e3 * sum(timed) / len(timed), "last_logits": logits}
 
 
 def run_reference(args):
@@ -172,6 +212,8 @@ def run_reference(args):
     steps = max(1, args.steps)            # one step = one reference mini-batch of 32 pairs (about 1 s on 16 cores)
     warm = max(1, args.warmup)
     cb = cpu_baseline(args, cfg, news, imp, sd, steps=steps, warmup=warm)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": cb["last_logits"].numpy()})
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
             "steps": steps, "warmup": warm, "ms_per_step": cb["ms_per_step"], "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -383,12 +425,16 @@ def run_b200(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(args.steps):
-            _, _, _, sums = step()
+            last_scores, _, last_per_imp, sums = step()
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
         launches = int(lib.lime_launch_count())
         result = sums.tolist()
+        if args.dump_outputs and rank == 0:      # before the passes below reuse the scores buffer
+            dump_outputs(args.dump_outputs, {"scores": last_scores.cpu().numpy(),
+                                             "per_impression_metrics": last_per_imp.cpu().numpy(),
+                                             "metric_sums": sums.cpu().numpy()})
         fallback_units = int(dimp.work_counter[1])      # units of the last timed step that the exact kernel re-scored
         # ---- the dominant kernel alone (roofline numerator) ----
         k0, k1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
