@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define LIME_B200_ABI_VERSION 4
+#define LIME_B200_ABI_VERSION 5
 
 /* Compile-time model geometry of the LIME-CROWN-CROWN configuration (config.py:54-91 defaults). */
 #define LIME_D        400   /* lime_output_dim == news_embedding_dim == attention_dim          */
@@ -337,6 +337,27 @@ int lime_rank_metrics(const float *scores, const uint8_t *labels, const int64_t 
 /* sums[0..3] = sum over valid impressions of the 4 metrics, sums[4] = number of valid impressions
  * (deterministic fixed-order reduction; the caller divides, or all-reduces across ranks first).  */
 int lime_metrics_reduce(const double *metrics, int64_t num_impressions, double *sums, void *stream);
+
+/* ---- top-k news of a pool per user (recommend.top_k; csrc/topk.cu) ---------------------------
+ * Top-k of every user's scores over a news pool.
+ * scores [users, pool] fp32: row u = user u's scores in PLAN order (position c of the pool plan).
+ * pool_index [pool] int32: the caller's index of plan position c (output id and tie-break key).
+ * pool_news [pool] int32: cache row of position c (used only for the clicked-history exclusion).
+ * exclude [pool] uint8 or NULL: nonzero = never returned (expired news, caller filters).
+ * hist_news / hist_mask [users, max_history] or NULL: a position whose pool_news equals a masked-in history
+ *   slot of user u is never returned to u (padding slots, mask 0, exclude nothing).
+ * Order: descending score; equal scores (-0.0 == +0.0) by ascending pool_index -- the order of
+ *   lime_rank_metrics on the pool in the caller's order.  NaN scores are never returned.
+ * out_index [users, k] int32 (caller's pool index, -1 past out_count), out_score [users, k] fp32 (-inf past
+ *   out_count), out_count [users] int32 = min(k, returnable positions).  1 <= k <= LIME_TOPK_MAX (1024).
+ *   A returned -0.0 score reads +0.0.
+ * scratch: caller-owned device buffer of lime_pool_topk_scratch_bytes(users, pool, k) bytes (0: may be NULL). */
+#define LIME_TOPK_MAX 1024
+int64_t lime_pool_topk_scratch_bytes(int32_t users, int64_t pool, int32_t k);
+int     lime_pool_topk(const float *scores, int32_t users, int64_t pool, const int32_t *pool_index,
+                       const int32_t *pool_news, const uint8_t *exclude, const int32_t *hist_news,
+                       const uint8_t *hist_mask, int32_t max_history, int32_t k, int32_t *out_index,
+                       float *out_score, int32_t *out_count, void *scratch, void *stream);
 
 
 /* ---- training: backward kernels of the same path (trainer.py:131-146 differentiates through them) ----

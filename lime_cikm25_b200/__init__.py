@@ -9,11 +9,11 @@ from . import _lib
 from . import attn_modules as layers
 from . import news_modules as newsEncoders
 from . import user_modules as userEncoders
-from . import engine, ops, synth, trainer, training, util
+from . import engine, ops, recommend, synth, trainer, training, util
 from .model import Model
 from .util import (NewsVectorCache, build_news_cache, compute_scores, evaluate_impressions,
                    score_impressions)
 
-__all__ = ["Model", "newsEncoders", "userEncoders", "layers", "util", "engine", "ops", "synth", "trainer", "training",
+__all__ = ["Model", "newsEncoders", "userEncoders", "layers", "util", "engine", "ops", "recommend", "synth", "trainer", "training",
            "NewsVectorCache", "build_news_cache", "compute_scores", "evaluate_impressions",
            "score_impressions"]

@@ -635,8 +635,92 @@ def build_units(cand_off, tile_c, cand_bp=None, triples=None, max_pairs=20):
     return np.asarray(ui, np.int64), np.asarray(up, np.int64), np.asarray(uc, np.int64)
 
 
+def plan_pool(bucket_pair, topic, limit):
+    """Work-unit plan of a news pool scored against every user (torch, CPU or device).  bucket_pair [C] (the approximate
+    (freshness, lifetime) bucket pair of _host_bucket_pairs) and topic [C] (compact topic id) -> (order, unit_pair0,
+    unit_count), int64:
+      order       a permutation of the pool: stable sort by (bucket pair, topic);
+      unit_pair0  first plan position of every unit, unit_count its size: units never straddle a bucket-pair group and
+                  hold at most ``limit`` candidates.
+    A unit then carries one distinct bucket pair beside its <= limit candidates (the tensor-core kernel's 40 operand-row
+    triples fit 39), and candidates of one topic have one candidate-aware attention vector (DESIGN.md section 3c), so the
+    kernel's expansion around the unit's centre is exact and the unit stays off the exact-kernel fallback."""
+    bp, tp = bucket_pair.long(), topic.long()
+    C = bp.numel()
+    if C == 0:
+        e = torch.zeros(0, dtype=torch.long, device=bp.device)
+        return e, e, e
+    order = torch.sort((bp << 32) | tp, stable=True).indices
+    sbp = bp[order]
+    pos = torch.arange(C, device=bp.device)
+    start = torch.ones(C, dtype=torch.bool, device=bp.device)
+    start[1:] = sbp[1:] != sbp[:-1]
+    first = torch.cummax(torch.where(start, pos, torch.zeros_like(pos)), 0).values     # first position of the group
+    unit_pair0 = torch.nonzero((pos - first) % int(limit) == 0).squeeze(1)
+    unit_count = torch.diff(unit_pair0, append=torch.tensor([C], device=bp.device))
+    return order, unit_pair0, unit_count
+
+
+class PoolPlan:
+    """A news pool laid out for lime_score_impressions (recommend.plan builds it).  Device tensors, all in plan order:
+    news / fresh / life [C] (cache row, seconds), remaining [C] or None (the remaining lifetime of lifetime_type 'fixed' /
+    'topic_wise'), index [C] int32 (the caller's index of the position), exclude [C] uint8 or None, bucket_pair / topic
+    [C] (the sort keys), and caller_news [C] int64 (the cache row of every caller index)."""
+
+    def __init__(self, news, fresh, life, remaining, index, exclude, bucket_pair, topic, caller_news):
+        self.news, self.fresh, self.life, self.remaining = news, fresh, life, remaining
+        self.index, self.exclude, self.bucket_pair, self.topic = index, exclude, bucket_pair, topic
+        self.caller_news = caller_news
+        self.device = news.device
+        self.templates = {}          # limit -> (unit_pair0, unit_count) int32 of one user
+
+    @property
+    def size(self):
+        return int(self.news.numel())
+
+    def units(self, limit):
+        """The unit template of one user for at most ``limit`` candidates per unit (the plan order is plan_pool's)."""
+        if limit not in self.templates:
+            _, p0, cnt = plan_pool(self.bucket_pair, self.topic, limit)
+            self.templates[limit] = (p0.to(torch.int32), cnt.to(torch.int32))
+        return self.templates[limit]
+
+
 class DeviceImpressions:
     """Impression set resident in HBM + the work-unit list of the scoring kernel."""
+
+    @classmethod
+    def from_pool(cls, plan, hist_news, hist_mask, hist_fresh, hist_life):
+        """Every one of Ub users (histories [Ub, H], device tensors) against the whole pool of ``plan`` (a PoolPlan): impression
+        u = user u, its candidates the pool in plan order (pair u * C + c).  Device tensors only, no host copies: the
+        candidate arrays are expanded copies of the plan's, the unit list is the plan's template shifted by u * C.
+        H <= 56 runs the tensor-core kernel; longer histories (up to 224) run the exact kernel, because the chunked
+        tensor-core path (DeviceImpressions.chunked) is built from host arrays -- correct, but several times slower."""
+        self = cls.__new__(cls)
+        dev = hist_mask.device
+        Ub, H = hist_mask.shape
+        C = plan.size
+        if Ub * C >= 2 ** 31:
+            raise _lib.LimeError("from_pool: %d users x %d news exceed the int32 pair index" % (Ub, C))
+        i32 = dict(dtype=torch.int32, device=dev)
+        self.tile_c = choose_tile_c(H)
+        p0, cnt = plan.units(min(self.tile_c, TC_TRIPLES - 2))     # room for one bucket-pair knife-edge per unit
+        nu = p0.numel()
+        self.max_history, self.num_pairs, self.num_impressions, self.num_units = H, Ub * C, Ub, Ub * nu
+        self.device = dev
+        self.planned_buckets = None
+        u = torch.arange(Ub, **i32).view(Ub, 1)
+        pairs = lambda t: t.view(1, C).expand(Ub, C).reshape(-1)
+        self.dev = dict(
+            hist_news=hist_news.to(torch.int32).contiguous(), hist_mask=hist_mask.to(torch.uint8).contiguous(),
+            hist_fresh=hist_fresh.float().contiguous(), hist_life=hist_life.float().contiguous(),
+            cand_news=pairs(plan.news), cand_fresh=pairs(plan.fresh), cand_life=pairs(plan.life),
+            unit_imp=u.expand(Ub, nu).reshape(-1), unit_pair0=(p0.view(1, nu) + u * C).reshape(-1),
+            unit_count=cnt.view(1, nu).expand(Ub, nu).reshape(-1))
+        if plan.remaining is not None:
+            self.dev["cand_remaining"] = pairs(plan.remaining)
+        self.work_counter = torch.zeros(int(_lib.load().lime_score_scratch_ints(self.num_units)), **i32)
+        return self
 
     @classmethod
     def from_pairs(cls, hist_mask, hist_fresh, hist_life, cand_fresh, cand_life, cand_remaining, n_cand):

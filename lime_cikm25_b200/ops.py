@@ -389,6 +389,42 @@ def rank_metrics(scores, labels, cand_off, want_ranks=True):
     return ranks, metrics
 
 
+TOPK_MAX = 1024      # LIME_TOPK_MAX
+
+
+def pool_topk(scores, k, pool_index, pool_news=None, exclude=None, hist_news=None, hist_mask=None):
+    """lime_pool_topk: scores [U, C] fp32 (row u = user u over the pool positions), pool_index [C] int32 (the id each
+    position returns and its tie-break key), optional pool_news [C] int32 + hist_news / hist_mask [U, H] int32 / uint8
+    (a position whose news is in the user's masked-in history is never returned), optional exclude [C] uint8.
+    -> (index [U, k] int32, -1 padded; score [U, k] fp32, -inf padded; count [U] int32): per user the k largest
+    scores, equal scores by ascending pool_index, NaN never returned."""
+    lib = _lib.require_device()
+    U, C = scores.shape
+    if not scores.is_contiguous():
+        raise ValueError("scores must be contiguous")
+    if pool_index.numel() != C or (pool_news is not None and pool_news.numel() != C) or (exclude is not None and exclude.numel() != C):
+        raise ValueError("pool arrays must have one entry per score column")
+    H = 0
+    if hist_news is not None:
+        if hist_mask is None or hist_news.dim() != 2 or hist_news.shape[0] != U or hist_mask.shape != hist_news.shape:
+            raise ValueError("hist_news / hist_mask must both be [users, max_history]")
+        if not (hist_news.is_contiguous() and hist_mask.is_contiguous()):
+            raise ValueError("hist_news / hist_mask must be contiguous")
+        H = hist_news.shape[1]
+    dev = scores.device
+    idx = torch.empty((U, k), dtype=torch.int32, device=dev)
+    val = torch.empty((U, k), dtype=torch.float32, device=dev)
+    cnt = torch.empty((U,), dtype=torch.int32, device=dev)
+    nbytes = int(lib.lime_pool_topk_scratch_bytes(U, C, int(k)))
+    scratch = torch.empty((nbytes,), dtype=torch.uint8, device=dev) if nbytes > 0 else None
+    check(lib.lime_pool_topk(_ptr(scores, torch.float32, "scores"), U, C, _ptr(pool_index, torch.int32, "pool_index"),
+                             _ptr(pool_news, torch.int32, "pool_news"), _ptr(exclude, torch.uint8, "exclude"),
+                             _ptr(hist_news, torch.int32, "hist_news"), _ptr(hist_mask, torch.uint8, "hist_mask"), H, int(k),
+                             idx.data_ptr(), val.data_ptr(), cnt.data_ptr(),
+                             scratch.data_ptr() if scratch is not None else None, _stream()), "lime_pool_topk")
+    return idx, val, cnt
+
+
 def metrics_reduce(metrics):
     """[I,4] fp64 -> fp64 [5] = (sum auc, sum mrr, sum ndcg5, sum ndcg10, valid impressions)."""
     lib = _lib.require_device()

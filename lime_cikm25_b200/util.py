@@ -198,6 +198,22 @@ def _read_truth(path, cand_off):
     return labels
 
 
+def remaining_lifetime(config, cand_fresh, cand_category):
+    """Remaining lifetime handed to RemainingLifetimeWeighting per candidate (util.py:98-104): fp32 [P] for
+    lifetime_type 'fixed' (fixed_lifetime - freshness) and 'topic_wise' (category_lifetime_map[category] - freshness),
+    None for 'user_topic' (the scoring kernel then uses lifetime - freshness).  cand_fresh: fp32 numpy [P];
+    cand_category: a callable returning the candidates' category ids (evaluated for 'topic_wise' only)."""
+    if config.lifetime_type == "fixed":                                     # util.py:98-99
+        return np.float32(config.fixed_lifetime) - cand_fresh
+    if config.lifetime_type == "topic_wise":                                # util.py:100-102
+        clm = config.category_lifetime_map
+        clm = clm.detach().cpu().numpy() if torch.is_tensor(clm) else np.asarray(clm)
+        return clm[cand_category()].astype(np.float32) - cand_fresh
+    if config.lifetime_type != "user_topic":
+        raise ValueError("Invalid lifetime_type")
+    return None
+
+
 def compute_scores(model, corpus, batch_size, mode, result_file, dataset):
     """Reference signature (util.py:77).  Builds the news-vector cache, scores every dev/test pair
     with the fused kernel, writes the rank file in the reference's format and returns
@@ -208,15 +224,7 @@ def compute_scores(model, corpus, batch_size, mode, result_file, dataset):
     news, imp = corpus_to_tables(corpus, mode)
     device = next(model.parameters()).device
     model.eval()
-    remaining = None
-    if config.lifetime_type == "fixed":                                     # util.py:98-99
-        remaining = np.float32(config.fixed_lifetime) - imp.cand_fresh
-    elif config.lifetime_type == "topic_wise":                              # util.py:100-102
-        clm = config.category_lifetime_map
-        clm = clm.detach().cpu().numpy() if torch.is_tensor(clm) else np.asarray(clm)
-        remaining = clm[news.category[imp.cand_news]].astype(np.float32) - imp.cand_fresh
-    elif config.lifetime_type != "user_topic":
-        raise ValueError("Invalid lifetime_type")
+    remaining = remaining_lifetime(config, imp.cand_fresh, lambda: news.category[imp.cand_news])
     labeled = dataset != "large" or mode != "test"
     if labeled:
         imp.labels = _read_truth(mode + "/ref/truth-%s.txt" % dataset, imp.cand_off)
