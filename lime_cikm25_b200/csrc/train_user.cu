@@ -35,6 +35,9 @@ __device__ __forceinline__ CaSmem ca_carve(float *sm, int N, int H) {
 __host__ __device__ inline size_t ca_smem_floats(int N, int H) {
     return (size_t)N * kUD + (size_t)H * kUD + (size_t)kUHeads * N * H + 2 * N + 2 * H + 8;
 }
+// Dynamic shared memory both directions admit: the 227 KB opt-in less 1 KB for the backward's static dagg / dqw / red arrays.
+// One limit for both, so that no (N, H) runs its forward and then fails in its backward.
+constexpr size_t kCaSmemLimit = 232448 - 1024;
 
 // forward pieces shared by the forward and backward kernels; on return P (before the dropout), qn, qw, agg, a are valid
 __device__ void ca_forward(const CaSmem &s, const float *__restrict__ Qp, const float *__restrict__ Kp,
@@ -433,7 +436,7 @@ extern "C" int lime_ca_attention_fwd(const float *Qp, const float *Kp, const uin
     LIME_CHECK_ARG(N >= 1 && N <= 64 && H >= 1 && H <= 64, "lime_ca_attention_fwd: N=%d, H=%d must be in [1,64]", N, H);
     if (B <= 0) return 0;
     const size_t smem = sizeof(float) * ca_smem_floats(N, H);
-    LIME_CHECK_ARG(smem <= 232448, "lime_ca_attention_fwd: N=%d, H=%d needs %zu B of shared memory", N, H, smem);
+    LIME_CHECK_ARG(smem <= kCaSmemLimit, "lime_ca_attention_fwd: N=%d, H=%d needs %zu B of shared memory", N, H, smem);
     LIME_CUDA(cudaFuncSetAttribute(ca_attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     ca_attn_fwd_kernel<<<B, 256, smem, as_stream(stream)>>>(Qp, Kp, mask, N, H, 1.0f / sqrtf((float)kUD), p_drop, seed, a);
     LIME_LAUNCH_CHECK("ca_attn_fwd_kernel");
@@ -446,7 +449,7 @@ extern "C" int lime_ca_attention_bwd(const float *Qp, const float *Kp, const uin
     LIME_CHECK_ARG(N >= 1 && N <= 64 && H >= 1 && H <= 64, "lime_ca_attention_bwd: N=%d, H=%d must be in [1,64]", N, H);
     if (B <= 0) return 0;
     const size_t smem = sizeof(float) * ca_smem_floats(N, H);
-    LIME_CHECK_ARG(smem <= 232448 - 1024, "lime_ca_attention_bwd: N=%d, H=%d needs %zu B of shared memory", N, H, smem);
+    LIME_CHECK_ARG(smem <= kCaSmemLimit, "lime_ca_attention_bwd: N=%d, H=%d needs %zu B of shared memory", N, H, smem);
     LIME_CUDA(cudaFuncSetAttribute(ca_attn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     ca_attn_bwd_kernel<<<B, 256, smem, as_stream(stream)>>>(Qp, Kp, mask, N, H, 1.0f / sqrtf((float)kUD), p_drop, seed, da, dQp, dKp);
     LIME_LAUNCH_CHECK("ca_attn_bwd_kernel");

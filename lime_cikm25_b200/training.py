@@ -8,8 +8,8 @@ applies inverted dropout at the SAME sites with its own stateless counter-based 
 re-evaluates the forward's mask): word embeddings, after the positional encoding, inside
 nn.TransformerEncoderLayer (attention weights, after out_proj, after the FFN activation, after linear2),
 category embeddings, the fixed p = 0.2 on the candidate-aware attention weights (layers.py:36,74) and the
-user-node rows.  Gradient parity is tested with every p = 0 (SURVEY.md section 7), the masks by their
-statistics (tests/test_gpu_training.py).
+user-node rows.  Gradient parity is tested with every p = 0 (SURVEY.md section 7, tests/test_gpu_training.py)
+and with every site live, against the oracle under the same masks (tests/test_gpu_training_parity.py).
 """
 from __future__ import annotations
 

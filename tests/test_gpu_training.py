@@ -135,7 +135,9 @@ def test_training_step_gradients(lib, bs, B):
     """Model.forward in training mode (B samples x (50 history + 5 candidates)), the reference trainer's
     loss (trainer.py:71-73) and backward(): logits and EVERY trainable parameter's gradient vs fp64
     autograd through the oracle (itself pinned to the reference's autograd in
-    tests/test_oracle_vs_reference.py).  bs = 64 > H: user-node rows enter the GraphSAGE mean."""
+    tests/test_oracle_vs_reference.py).  The GraphSAGE prefix is the runtime batch B (3 or 4 < H = 50), so no
+    user-node row enters the mean here, whatever config.batch_size is: tests/test_gpu_training_parity.py runs a step
+    with B > H."""
     cfg, model, sd = _make(31, batch_size=bs)
     news = synth.make_news_table(40, vocabulary_size=cfg.vocabulary_size, seed=4)
     batch = synth.make_train_batch(news, B, seed=6)
