@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define LIME_B200_ABI_VERSION 5
+#define LIME_B200_ABI_VERSION 6
 
 /* Compile-time model geometry of the LIME-CROWN-CROWN configuration (config.py:54-91 defaults). */
 #define LIME_D        400   /* lime_output_dim == news_embedding_dim == attention_dim          */
@@ -358,6 +358,33 @@ int     lime_pool_topk(const float *scores, int32_t users, int64_t pool, const i
                        const int32_t *pool_news, const uint8_t *exclude, const int32_t *hist_news,
                        const uint8_t *hist_mask, int32_t max_history, int32_t k, int32_t *out_index,
                        float *out_score, int32_t *out_count, void *scratch, void *stream);
+
+/* ---- rank of held-out clicks in the whole pool (recommend.evaluate; csrc/topk.cu) -----------
+ * For each user u: the rank of every target among the positions lime_pool_topk could return to u, and ranking
+ * metrics of the ranked targets.  scores / pool_index / pool_news / exclude / hist_news / hist_mask / max_history
+ * as in lime_pool_topk (pool_news is required only with hist_news).
+ * Eligible positions: not marked by exclude, score not NaN, and (with hist_news) news not in u's masked-in history.
+ *   They are ordered by lime_pool_topk's key: score descending (-0.0 == +0.0), then ascending pool_index.
+ * target_pos [users, targets] int32: pool positions (plan order) of u's held-out clicks; -1 (or any value outside
+ *   [0, pool)) = no target.  1 <= targets <= LIME_POOL_RANK_MAX_TARGETS.
+ * out_rank [users, targets] int32: 1-based position of the target in u's order, counting every eligible position
+ *   (other targets included), so rank r <= k means lime_pool_topk(k) returns it at position r.  0 = unranked: no
+ *   target, an ineligible position, or a second or later copy of a position already listed for u.
+ * out_ranked [users] int32 = n, the ranked targets; out_eligible [users] int64 = N, the eligible positions.
+ * out_metrics [users, 4 + 2 * num_cutoffs] fp64 = auc, mrr, ndcg5, ndcg10, then recall@K, ndcg@K per cutoff K:
+ *   auc = (sum (N - r_i) - n(n-1)/2) / (n (N - n)) (integer numerator; NaN when N == n), mrr = mean 1/r_i,
+ *   ndcg@K = sum_{r_i <= K} 1/log2(r_i + 1) over the ideal sum_{i <= min(n, K)} 1/log2(i + 1), recall@K =
+ *   #{r_i <= K} / n -- the formulas of lime_rank_metrics.  n == 0: an all-NaN row.
+ * cutoffs: HOST array of num_cutoffs (<= LIME_POOL_RANK_MAX_CUTOFFS) values >= 1, passed by value into the launch.
+ * scratch: caller-owned device buffer of lime_pool_rank_scratch_bytes(users, targets) bytes; zeroed here on `stream`. */
+#define LIME_POOL_RANK_MAX_TARGETS 256
+#define LIME_POOL_RANK_MAX_CUTOFFS 8
+int64_t lime_pool_rank_scratch_bytes(int32_t users, int32_t targets);
+int     lime_pool_rank_metrics(const float *scores, int32_t users, int64_t pool, const int32_t *pool_index,
+                               const int32_t *pool_news, const uint8_t *exclude, const int32_t *hist_news,
+                               const uint8_t *hist_mask, int32_t max_history, const int32_t *target_pos, int32_t targets,
+                               const int32_t *cutoffs, int32_t num_cutoffs, int32_t *out_rank, int32_t *out_ranked,
+                               int64_t *out_eligible, double *out_metrics, void *scratch, void *stream);
 
 
 /* ---- training: backward kernels of the same path (trainer.py:131-146 differentiates through them) ----

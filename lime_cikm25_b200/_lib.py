@@ -91,6 +91,8 @@ PROTOTYPES = {
     "lime_metrics_reduce": (C.c_int, [P, I64, P, P]),
     "lime_pool_topk_scratch_bytes": (I64, [I32, I64, I32]),
     "lime_pool_topk": (C.c_int, [P, I32, I64, P, P, P, P, P, I32, I32, P, P, P, P, P]),
+    "lime_pool_rank_scratch_bytes": (I64, [I32, I32]),
+    "lime_pool_rank_metrics": (C.c_int, [P, I32, I64, P, P, P, P, P, I32, P, I32, P, I32, P, P, P, P, P, P]),
     "lime_gemm": (C.c_int, [P, I64, C.c_int, P, I64, C.c_int, P, I64, I64, C.c_int, I64, F32, C.c_int, P]),
     "lime_gemm_bf16": (C.c_int, [P, I64, C.c_int, P, I64, C.c_int, P, I64, I64, C.c_int, I64, F32, C.c_int, P]),
     "lime_gemm_bf16_tn_tma": (C.c_int, [P, I64, P, I64, P, I64, I32, I32, I64, F32, I32, P]),
@@ -125,7 +127,7 @@ PROTOTYPES = {
     "lime_click_score_bwd": (C.c_int, [P, P, P, P, I64, P, P, P]),
 }
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 _lib = None
 
 

@@ -56,6 +56,16 @@ __device__ __forceinline__ float warp_max(float v) {
     for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
     return v;
 }
+__device__ __forceinline__ double warp_sum_d(double v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+__device__ __forceinline__ long long warp_sum_ll(long long v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
 
 // Stateless counter-based generator of the training dropouts: (seed, element index) -> 32 random bits via two rounds of a
 // 64-bit mix; forward and backward evaluate the same mask.  drop_scale = keep / (1 - p).

@@ -12,17 +12,6 @@ namespace lime {
 
 constexpr int kMetricWarps = 4;
 
-__device__ __forceinline__ double warp_sum_d(double v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-__device__ __forceinline__ long long warp_sum_ll(long long v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-
 __global__ void __launch_bounds__(kMetricWarps * 32)
 rank_metrics_kernel(const float *__restrict__ scores, const uint8_t *__restrict__ labels,
                     const int64_t *__restrict__ cand_off, int64_t num_impressions,

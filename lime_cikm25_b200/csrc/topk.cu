@@ -38,6 +38,56 @@ __device__ __forceinline__ float ord_score(uint32_t o) {
     return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
 }
 
+__device__ __forceinline__ uint64_t pool_key(float s, int32_t pool_index) {
+    return ((uint64_t)score_ord(s) << 32) | (uint32_t)~(uint32_t)pool_index;
+}
+
+// The masked-in history ids of user u, sorted ascending into hsorted[0, nh); returns nh.  Every thread of a
+// kTopkThreads-thread CTA calls (it synchronises); *s_nh must be 0 and visible to all threads on entry.
+__device__ __forceinline__ int load_history(const int32_t *__restrict__ hist_news, const uint8_t *__restrict__ hist_mask,
+                                            int max_history, int64_t u, int *hraw, int *hsorted, int *s_nh) {
+    const int tid = threadIdx.x;
+    for (int h0 = 0; h0 < max_history; h0 += kTopkThreads) {       // masked-in ids of the history, then rank-sorted
+        const int h = h0 + tid;
+        const bool ok = h < max_history && hist_mask[u * max_history + h] != 0;
+        const unsigned m = __ballot_sync(0xffffffffu, ok);
+        if (m) {
+            const int lane = tid & 31, leader = __ffs(m) - 1;
+            int base = 0;
+            if (lane == leader) base = atomicAdd(s_nh, __popc(m));
+            base = __shfl_sync(0xffffffffu, base, leader);
+            if (ok) hraw[base + __popc(m & ((1u << lane) - 1u))] = hist_news[u * max_history + h];
+        }
+    }
+    __syncthreads();
+    const int nh = *s_nh;
+    for (int t = tid; t < nh; t += kTopkThreads) {
+        const int v = hraw[t];
+        int r = 0;
+        for (int j = 0; j < nh; ++j) r += hraw[j] < v || (hraw[j] == v && j < t);
+        hsorted[r] = v;
+    }
+    __syncthreads();
+    return nh;
+}
+
+// The exclusion test: may pool position i with score s be returned to the user whose sorted history is hsorted[0, nh)?
+// Not NaN, not excluded, and its news not clicked (binary search; nh == 0 skips it).
+__device__ __forceinline__ bool returnable(float s, int64_t i, const uint8_t *__restrict__ exclude,
+                                           const int32_t *__restrict__ pool_news, const int *hsorted, int nh) {
+    bool ok = s == s && !(exclude != nullptr && exclude[i]);
+    if (ok && nh > 0) {
+        const int nw = pool_news[i];
+        int a = 0, b = nh;                    // first slot >= nw
+        while (a < b) {
+            const int mid = (a + b) >> 1;
+            if (hsorted[mid] < nw) a = mid + 1; else b = mid;
+        }
+        ok = !(a < nh && hsorted[a] == nw);
+    }
+    return ok;
+}
+
 // Block-wide append of `key` where `ok`; every lane of the warp must call (the loop bounds below are warp-uniform).
 // Appends past `cap` are dropped (only reachable with duplicate pool_index values).
 __device__ __forceinline__ void append_key(bool ok, uint64_t key, uint64_t *buf, int *count, int cap) {
@@ -79,30 +129,7 @@ pool_topk_kernel(const float *__restrict__ scores, const uint64_t *__restrict__ 
     if (tid == 0) { s_nh = 0; s_n = 0; s_nsel = 0; }
     __syncthreads();
 
-    int nh = 0;
-    if (kScores && hist_news != nullptr) {
-        for (int h0 = 0; h0 < max_history; h0 += kTopkThreads) {     // masked-in ids of the history, then rank-sorted
-            const int h = h0 + tid;
-            const bool ok = h < max_history && hist_mask[u * max_history + h] != 0;
-            const unsigned m = __ballot_sync(0xffffffffu, ok);
-            if (m) {
-                const int lane = tid & 31, leader = __ffs(m) - 1;
-                int base = 0;
-                if (lane == leader) base = atomicAdd(&s_nh, __popc(m));
-                base = __shfl_sync(0xffffffffu, base, leader);
-                if (ok) hraw[base + __popc(m & ((1u << lane) - 1u))] = hist_news[u * max_history + h];
-            }
-        }
-        __syncthreads();
-        nh = s_nh;
-        for (int t = tid; t < nh; t += kTopkThreads) {
-            const int v = hraw[t];
-            int r = 0;
-            for (int j = 0; j < nh; ++j) r += hraw[j] < v || (hraw[j] == v && j < t);
-            hsorted[r] = v;
-        }
-        __syncthreads();
-    }
+    const int nh = kScores && hist_news != nullptr ? load_history(hist_news, hist_mask, max_history, u, hraw, hsorted, &s_nh) : 0;
 
     // ---- load: one read per input, keys compacted into shared memory ----
     for (int64_t i0 = lo; i0 < hi; i0 += kTopkThreads) {
@@ -112,17 +139,8 @@ pool_topk_kernel(const float *__restrict__ scores, const uint64_t *__restrict__ 
         if (i < hi) {
             if (kScores) {
                 const float s = scores[u * n_in + i];
-                ok = s == s && !(exclude != nullptr && exclude[i]);
-                if (ok && nh > 0) {
-                    const int nw = pool_news[i];
-                    int a = 0, b = nh;                    // first slot >= nw
-                    while (a < b) {
-                        const int mid = (a + b) >> 1;
-                        if (hsorted[mid] < nw) a = mid + 1; else b = mid;
-                    }
-                    ok = !(a < nh && hsorted[a] == nw);
-                }
-                if (ok) key = ((uint64_t)score_ord(s) << 32) | (uint32_t)~(uint32_t)pool_index[i];
+                ok = returnable(s, i, exclude, pool_news, hsorted, nh);
+                if (ok) key = pool_key(s, pool_index[i]);
             } else {
                 key = keys_in[u * n_in + i];
                 ok = key != 0;
@@ -236,6 +254,208 @@ static TopkPlan topk_plan(int32_t users, int64_t pool, int32_t k) {
     return p;
 }
 
+
+// ---- ranks of held-out clicks in the whole pool (lime_pool_rank_metrics) ----------------------------------------------
+// Count launch: CTA blockIdx.x = u * groups + g over positions [g * slice, (g + 1) * slice) of user u (round 0's groups).
+// It builds u's n <= T target keys (eligible, first copy of each position) sorted ascending in shared memory, then
+// reads every score of its slice once: an eligible position with key x adds 1 to bin p = #{targets with key < x}
+// (p = 0, a position below every target, costs no atomic).  Target j (0-based ascending) then has rank
+// 1 + sum_{p > j} bin[p]: the eligible positions above it.  counts[u * (T + 1)] = eligible positions, counts[.. + p] =
+// bin p; slot_order[u * T + t] = ascending index of target slot t, -1 = unranked (written by group 0).
+constexpr int kRankThreads = kTopkThreads;      // load_history's CTA size
+constexpr int kRankMaxT = LIME_POOL_RANK_MAX_TARGETS;
+constexpr int kFinishWarps = 4;
+constexpr int kMaxColumnsK = 2 + LIME_POOL_RANK_MAX_CUTOFFS;      // nDCG cutoffs 5, 10, then the caller's
+
+struct RankCutoffs {
+    int32_t k[LIME_POOL_RANK_MAX_CUTOFFS];
+    int32_t n;
+};
+
+__global__ void __launch_bounds__(kRankThreads)
+pool_rank_count_kernel(const float *__restrict__ scores, int64_t pool, int32_t slice, int32_t groups,
+                       const int32_t *__restrict__ pool_index, const int32_t *__restrict__ pool_news,
+                       const uint8_t *__restrict__ exclude, const int32_t *__restrict__ hist_news,
+                       const uint8_t *__restrict__ hist_mask, int32_t max_history, const int32_t *__restrict__ target_pos,
+                       int32_t T, unsigned *__restrict__ counts, int32_t *__restrict__ slot_order) {
+    __shared__ int hraw[kHistMax], hsorted[kHistMax];
+    __shared__ uint64_t tkey[kRankMaxT], tsorted[kRankMaxT];
+    __shared__ int tpos[kRankMaxT];
+    __shared__ unsigned bins[kRankMaxT + 1];
+    __shared__ int s_nh, s_n;
+    __shared__ unsigned s_elig;
+
+    const int tid = threadIdx.x, lane = tid & 31;
+    const int64_t u = blockIdx.x / groups;
+    const int g = (int)(blockIdx.x - u * groups);
+    const int64_t lo = (int64_t)g * slice;
+    const int64_t hi = min(pool, lo + slice);
+    const float *row = scores + u * pool;
+    if (tid == 0) { s_nh = 0; s_n = 0; s_elig = 0; }
+    for (int b = tid; b <= T; b += kRankThreads) bins[b] = 0;
+    __syncthreads();
+    const int nh = hist_news != nullptr ? load_history(hist_news, hist_mask, max_history, u, hraw, hsorted, &s_nh) : 0;
+
+    // ---- targets: key of every eligible slot, later copies of a position dropped, rank-sorted ascending ----
+    uint64_t key = 0;
+    int pos = -1;
+    if (tid < T) {
+        pos = target_pos[u * T + tid];
+        if (pos >= 0 && pos < pool) {
+            const float s = row[pos];
+            if (returnable(s, pos, exclude, pool_news, hsorted, nh)) key = pool_key(s, pool_index[pos]);
+        }
+        if (key == 0) pos = -1;
+        tpos[tid] = pos;
+    }
+    __syncthreads();
+    if (key != 0)
+        for (int j = 0; j < tid; ++j)
+            if (tpos[j] == pos) { key = 0; break; }
+    if (tid < T) tkey[tid] = key;
+    __syncthreads();
+    int r = -1;
+    if (key != 0) {
+        r = 0;
+        for (int j = 0; j < T; ++j) r += tkey[j] != 0 && tkey[j] < key;
+        tsorted[r] = key;
+        atomicAdd(&s_n, 1);
+    }
+    if (g == 0 && tid < T) slot_order[u * T + tid] = r;
+    __syncthreads();
+    const int n = s_n;
+    const uint32_t lowest = n > 0 ? (uint32_t)(tsorted[0] >> 32) : 0xffffffffu;
+
+    // ---- positions: eligible count, and bin p of every eligible position above p targets ----
+    unsigned elig = 0;
+    for (int64_t i0 = lo; i0 < hi; i0 += kRankThreads) {
+        const int64_t i = i0 + tid;
+        int p = 0;
+        if (i < hi) {
+            const float s = row[i];
+            if (returnable(s, i, exclude, pool_news, hsorted, nh)) {
+                ++elig;
+                if (n > 0 && score_ord(s) >= lowest) {  // else below every target: p = 0 without reading pool_index
+                    const uint64_t x = pool_key(s, pool_index[i]);
+                    int a = 0, b = n;                   // p = first slot >= x
+                    while (a < b) {
+                        const int mid = (a + b) >> 1;
+                        if (tsorted[mid] < x) a = mid + 1; else b = mid;
+                    }
+                    p = a;
+                }
+            }
+        }
+        // warp-aggregated increments: a low-ranked target sends most of the pool into one bin
+        if (__any_sync(0xffffffffu, p > 0)) {
+            const unsigned peers = __match_any_sync(0xffffffffu, p);
+            if (p > 0 && lane == __ffs(peers) - 1) atomicAdd(&bins[p], (unsigned)__popc(peers));
+        }
+    }
+    elig = __reduce_add_sync(0xffffffffu, elig);
+    if (lane == 0 && elig) atomicAdd(&s_elig, elig);
+    __syncthreads();
+    unsigned *c = counts + u * (T + 1);
+    if (tid == 0 && s_elig) atomicAdd(c, s_elig);
+    for (int b = 1 + tid; b <= n; b += kRankThreads)
+        if (bins[b]) atomicAdd(c + b, bins[b]);
+}
+
+
+// Finish launch: one warp per user.  Ranks by a suffix sum over the bins (lane l owns bins 8l + 1 .. 8l + 8), written back
+// in the caller's slot order; then the counts and the metrics row (lime_rank_metrics' formulas, fp64).
+__global__ void __launch_bounds__(kFinishWarps * 32)
+pool_rank_finish_kernel(const unsigned *__restrict__ counts, const int32_t *__restrict__ slot_order, int32_t users,
+                        int32_t T, RankCutoffs cut, int32_t *__restrict__ out_rank, int32_t *__restrict__ out_ranked,
+                        int64_t *__restrict__ out_eligible, double *__restrict__ out_metrics) {
+    __shared__ int srank[kFinishWarps][kRankMaxT];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int64_t u = (int64_t)blockIdx.x * kFinishWarps + w;
+    if (u >= users) return;
+    const unsigned *c = counts + u * (T + 1);
+    const int32_t *slot = slot_order + u * T;
+    int n = 0;
+    for (int t = lane; t < T; t += 32) n += slot[t] >= 0;
+    n = __reduce_add_sync(0xffffffffu, n);
+    const long long N = c[0];
+
+    constexpr int kPer = kRankMaxT / 32;
+    unsigned v[kPer], tot = 0;
+#pragma unroll
+    for (int m = 0; m < kPer; ++m) {
+        const int b = lane * kPer + m + 1;
+        v[m] = b <= n ? c[b] : 0u;
+        tot += v[m];
+    }
+    unsigned above = tot;                               // inclusive suffix over lanes >= this one
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const unsigned x = __shfl_down_sync(0xffffffffu, above, o);
+        if (lane + o < 32) above += x;
+    }
+    above -= tot;
+#pragma unroll
+    for (int m = kPer - 1; m >= 0; --m) {              // target j = lane * kPer + m: 1 + bins j + 1 .. n
+        above += v[m];
+        if (lane * kPer + m < n) srank[w][lane * kPer + m] = 1 + (int)above;
+    }
+    __syncwarp();
+    for (int t = lane; t < T; t += 32) {
+        const int o = slot[t];
+        out_rank[u * T + t] = o >= 0 ? srank[w][o] : 0;
+    }
+
+    const int ncol = 2 + cut.n;
+    double *out = out_metrics + u * (4 + 2 * cut.n);
+    if (lane == 0) {
+        out_ranked[u] = n;
+        out_eligible[u] = N;
+    }
+    if (n == 0) {
+        for (int q = lane; q < 4 + 2 * cut.n; q += 32) out[q] = __longlong_as_double(0x7ff8000000000000LL);
+        return;
+    }
+    long long below = 0;                                // sum over targets of N - r
+    double rr = 0.0, dcg[kMaxColumnsK], ideal[kMaxColumnsK];
+    int hits[kMaxColumnsK];
+#pragma unroll
+    for (int q = 0; q < kMaxColumnsK; ++q) { dcg[q] = 0.0; ideal[q] = 0.0; hits[q] = 0; }
+    for (int j = lane; j < n; j += 32) {
+        const int r = srank[w][j];
+        below += N - r;
+        rr += 1.0 / (double)r;
+        const double gr = 1.0 / log2((double)r + 1.0);
+        const double gi = 1.0 / log2((double)(j + 1) + 1.0);     // ideal: the ranked targets at 1 .. n
+#pragma unroll
+        for (int q = 0; q < kMaxColumnsK; ++q) {
+            const int K = q == 0 ? 5 : q == 1 ? 10 : (q < ncol ? cut.k[q - 2] : 0);
+            if (r <= K) { dcg[q] += gr; hits[q] += 1; }
+            if (j + 1 <= K) ideal[q] += gi;
+        }
+    }
+    below = warp_sum_ll(below);
+    rr = warp_sum_d(rr);
+#pragma unroll
+    for (int q = 0; q < kMaxColumnsK; ++q) {
+        dcg[q] = warp_sum_d(dcg[q]);
+        ideal[q] = warp_sum_d(ideal[q]);
+        hits[q] = __reduce_add_sync(0xffffffffu, hits[q]);
+    }
+    if (lane == 0) {
+        const long long nn = n;
+        out[0] = (double)(below - nn * (nn - 1) / 2) / ((double)nn * (double)(N - nn));     // NaN when N == n
+        out[1] = rr / (double)nn;
+        out[2] = dcg[0] / ideal[0];
+        out[3] = dcg[1] / ideal[1];
+#pragma unroll
+        for (int q = 2; q < kMaxColumnsK; ++q)
+            if (q < ncol) {
+                out[4 + 2 * (q - 2)] = (double)hits[q] / (double)nn;
+                out[5 + 2 * (q - 2)] = dcg[q] / ideal[q];
+            }
+    }
+}
+
 }  // namespace lime
 
 using namespace lime;
@@ -291,5 +511,51 @@ extern "C" int lime_pool_topk(const float *scores, int32_t users, int64_t pool, 
         groups = next;
         uint64_t *t = in; in = out; out = t;
     }
+    return 0;
+}
+
+extern "C" int64_t lime_pool_rank_scratch_bytes(int32_t users, int32_t targets) {
+    if (users <= 0 || targets < 1 || targets > LIME_POOL_RANK_MAX_TARGETS) return 0;
+    return (int64_t)users * (2 * targets + 1) * (int64_t)sizeof(int32_t);   // counts [users, T + 1], slot_order [users, T]
+}
+
+extern "C" int lime_pool_rank_metrics(const float *scores, int32_t users, int64_t pool, const int32_t *pool_index,
+                                      const int32_t *pool_news, const uint8_t *exclude, const int32_t *hist_news,
+                                      const uint8_t *hist_mask, int32_t max_history, const int32_t *target_pos, int32_t targets,
+                                      const int32_t *cutoffs, int32_t num_cutoffs, int32_t *out_rank, int32_t *out_ranked,
+                                      int64_t *out_eligible, double *out_metrics, void *scratch, void *stream) {
+    LIME_CHECK_ARG(targets >= 1 && targets <= LIME_POOL_RANK_MAX_TARGETS, "lime_pool_rank_metrics: targets=%d not in [1, %d]",
+                   targets, LIME_POOL_RANK_MAX_TARGETS);
+    LIME_CHECK_ARG(scores && pool_index && target_pos && out_rank && out_ranked && out_eligible && out_metrics && scratch,
+                   "lime_pool_rank_metrics: null argument");
+    LIME_CHECK_ARG(num_cutoffs >= 0 && num_cutoffs <= LIME_POOL_RANK_MAX_CUTOFFS,
+                   "lime_pool_rank_metrics: num_cutoffs=%d not in [0, %d]", num_cutoffs, LIME_POOL_RANK_MAX_CUTOFFS);
+    LIME_CHECK_ARG(num_cutoffs == 0 || cutoffs != nullptr, "lime_pool_rank_metrics: null cutoffs");
+    RankCutoffs cut = {};
+    cut.n = num_cutoffs;
+    for (int q = 0; q < num_cutoffs; ++q) {
+        LIME_CHECK_ARG(cutoffs[q] >= 1, "lime_pool_rank_metrics: cutoff %d = %d < 1", q, cutoffs[q]);
+        cut.k[q] = cutoffs[q];
+    }
+    LIME_CHECK_ARG(users >= 0, "lime_pool_rank_metrics: users=%d < 0", users);
+    LIME_CHECK_ARG(pool >= 1 && pool < (1LL << 31), "lime_pool_rank_metrics: pool=%lld not in [1, 2^31)", (long long)pool);
+    LIME_CHECK_ARG((hist_news == nullptr) == (hist_mask == nullptr), "lime_pool_rank_metrics: hist_news and hist_mask go together");
+    LIME_CHECK_ARG(hist_news == nullptr || pool_news != nullptr, "lime_pool_rank_metrics: the clicked exclusion needs pool_news");
+    LIME_CHECK_ARG(hist_news == nullptr || (max_history >= 1 && max_history <= kHistMax),
+                   "lime_pool_rank_metrics: max_history=%d not in [1, %d]", max_history, kHistMax);
+    if (users == 0) return 0;
+    const TopkPlan p = topk_plan(users, pool, 1);       // round 0's groups: about 2 CTAs per SM even for one user
+    LIME_CHECK_ARG((int64_t)users * p.groups0 < (1LL << 31), "lime_pool_rank_metrics: users x groups exceeds the grid");
+    cudaStream_t st = as_stream(stream);
+    unsigned *counts = static_cast<unsigned *>(scratch);
+    int32_t *slot_order = reinterpret_cast<int32_t *>(counts + (int64_t)users * (targets + 1));
+    LIME_CUDA(cudaMemsetAsync(counts, 0, (size_t)users * (targets + 1) * sizeof(unsigned), st));
+    pool_rank_count_kernel<<<(unsigned)(users * p.groups0), kRankThreads, 0, st>>>(
+        scores, pool, p.slice0, (int32_t)p.groups0, pool_index, pool_news, exclude, hist_news, hist_mask, max_history,
+        target_pos, targets, counts, slot_order);
+    LIME_LAUNCH_CHECK("pool_rank_count_kernel");
+    pool_rank_finish_kernel<<<(unsigned)topk_cdiv(users, kFinishWarps), kFinishWarps * 32, 0, st>>>(
+        counts, slot_order, users, targets, cut, out_rank, out_ranked, out_eligible, out_metrics);
+    LIME_LAUNCH_CHECK("pool_rank_finish_kernel");
     return 0;
 }

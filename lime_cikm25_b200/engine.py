@@ -673,10 +673,19 @@ class PoolPlan:
         self.caller_news = caller_news
         self.device = news.device
         self.templates = {}          # limit -> (unit_pair0, unit_count) int32 of one user
+        self._positions = None
 
     @property
     def size(self):
         return int(self.news.numel())
+
+    def positions(self, news_num):
+        """[news_num] int32 device table: the plan position of every cache row, -1 = not in the pool (built once)."""
+        if self._positions is None or self._positions.numel() != news_num:
+            t = torch.full((news_num,), -1, dtype=torch.int32, device=self.device)
+            t[self.news.long()] = torch.arange(self.size, dtype=torch.int32, device=self.device)
+            self._positions = t
+        return self._positions
 
     def units(self, limit):
         """The unit template of one user for at most ``limit`` candidates per unit (the plan order is plan_pool's)."""

@@ -6,6 +6,8 @@ silently except where the docstring says so.
 """
 from __future__ import annotations
 
+import ctypes
+
 import torch
 
 from . import _lib
@@ -423,6 +425,50 @@ def pool_topk(scores, k, pool_index, pool_news=None, exclude=None, hist_news=Non
                              idx.data_ptr(), val.data_ptr(), cnt.data_ptr(),
                              scratch.data_ptr() if scratch is not None else None, _stream()), "lime_pool_topk")
     return idx, val, cnt
+
+
+POOL_RANK_MAX_TARGETS = 256      # LIME_POOL_RANK_MAX_TARGETS
+POOL_RANK_MAX_CUTOFFS = 8        # LIME_POOL_RANK_MAX_CUTOFFS
+
+
+def pool_rank_metrics(scores, pool_index, target_pos, cutoffs=(), pool_news=None, exclude=None, hist_news=None,
+                      hist_mask=None):
+    """lime_pool_rank_metrics: scores / pool_index / pool_news / exclude / hist_news / hist_mask as in pool_topk,
+    target_pos [U, T] int32 (pool positions of the held-out clicks, -1 = none), cutoffs a host sequence of ints >= 1.
+    -> (rank [U, T] int32, 0 = unranked; ranked [U] int32; eligible [U] int64; metrics [U, 4 + 2 len(cutoffs)] fp64 =
+    auc, mrr, ndcg5, ndcg10, recall@K, ndcg@K ...): the 1-based position of every target in the order pool_topk
+    returns, among every position it could return."""
+    lib = _lib.require_device()
+    U, C = scores.shape
+    if not scores.is_contiguous():
+        raise ValueError("scores must be contiguous")
+    if pool_index.numel() != C or (pool_news is not None and pool_news.numel() != C) or (exclude is not None and exclude.numel() != C):
+        raise ValueError("pool arrays must have one entry per score column")
+    if target_pos.dim() != 2 or target_pos.shape[0] != U or not target_pos.is_contiguous():
+        raise ValueError("target_pos must be a contiguous [users, targets] tensor")
+    H = 0
+    if hist_news is not None:
+        if hist_mask is None or hist_news.dim() != 2 or hist_news.shape[0] != U or hist_mask.shape != hist_news.shape:
+            raise ValueError("hist_news / hist_mask must both be [users, max_history]")
+        if not (hist_news.is_contiguous() and hist_mask.is_contiguous()):
+            raise ValueError("hist_news / hist_mask must be contiguous")
+        H = hist_news.shape[1]
+    T = target_pos.shape[1]
+    cut = [int(c) for c in cutoffs]
+    dev = scores.device
+    rank = torch.empty((U, T), dtype=torch.int32, device=dev)
+    ranked = torch.empty((U,), dtype=torch.int32, device=dev)
+    eligible = torch.empty((U,), dtype=torch.int64, device=dev)
+    metrics = torch.empty((U, 4 + 2 * len(cut)), dtype=torch.float64, device=dev)
+    scratch = torch.empty((max(1, int(lib.lime_pool_rank_scratch_bytes(U, T))),), dtype=torch.uint8, device=dev)
+    h_cut = (ctypes.c_int32 * max(1, len(cut)))(*cut)
+    check(lib.lime_pool_rank_metrics(_ptr(scores, torch.float32, "scores"), U, C, _ptr(pool_index, torch.int32, "pool_index"),
+                                     _ptr(pool_news, torch.int32, "pool_news"), _ptr(exclude, torch.uint8, "exclude"),
+                                     _ptr(hist_news, torch.int32, "hist_news"), _ptr(hist_mask, torch.uint8, "hist_mask"), H,
+                                     _ptr(target_pos, torch.int32, "target_pos"), T, h_cut, len(cut), rank.data_ptr(),
+                                     ranked.data_ptr(), eligible.data_ptr(), metrics.data_ptr(), scratch.data_ptr(), _stream()),
+          "lime_pool_rank_metrics")
+    return rank, ranked, eligible, metrics
 
 
 def metrics_reduce(metrics):

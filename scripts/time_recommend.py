@@ -1,6 +1,7 @@
-"""GPU: top-k recommendation over a news pool (recommend.plan / recommend.top_k), one JSON line per (pool, k).
+"""GPU: top-k recommendation over a news pool (recommend.plan / recommend.top_k), one JSON line per (pool, k), and its
+full-pool evaluation (recommend.evaluate), one JSON line per pool ("kind": "evaluate").
 
-    python scripts/time_recommend.py [--users 4096] [--pools all,16384,4096] [--ks 10,100] [--out FILE]
+    python scripts/time_recommend.py [--users 4096] [--pools all,16384,4096] [--ks 10,100] [--targets 8] [--out FILE]
 
 Workload: the 65,238-news cache of bench.py's MIND shape (BASELINE.json configs[1]), U histories from
 synth.make_impressions, a pool of every news or a random subset, freshness / lifetime drawn like synth's candidates.
@@ -13,6 +14,11 @@ Per configuration:
   topk_ms_per_launch      lime_pool_topk on that batch's scores (clicked exclusion on), torch_topk_ms torch.topk on the
                           same tensor
   users_per_s             recommend.top_k over all U users, end to end (scores, selection, id mapping)
+Evaluation, T targets per user drawn from the pool (cutoffs 10, 50, 100):
+  rank_ms_per_launch      lime_pool_rank_metrics (memset + count + finish) on the batch topk_ms_per_launch uses
+  rank_share_of_scoring   rank_ms_per_launch / score_ms_per_launch
+  eval_users_per_s        recommend.evaluate over all U users, end to end, alternated in the same process with
+                          recommend.top_k at k = 10 (topk_users_per_s)
 All times are CUDA events after a warm-up of every shape; the GPU name and power limit are read in the same process.
 """
 import argparse
@@ -79,6 +85,7 @@ def main():
     ap.add_argument("--users", type=int, default=4096)
     ap.add_argument("--pools", default="all,16384,4096")
     ap.add_argument("--ks", default="10,100")
+    ap.add_argument("--targets", type=int, default=8, help="held-out clicks per user of the evaluation pass")
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--out", default=None, help="also append the JSON lines to this file")
     args = ap.parse_args()
@@ -97,7 +104,14 @@ def main():
     hist = [torch.from_numpy(np.ascontiguousarray(a)).cuda() for a in (imp.hist_news, imp.hist_mask, imp.hist_fresh, imp.hist_life)]
     hist[1] = hist[1].to(torch.uint8)
     rng = np.random.default_rng(3)
+    trng = np.random.default_rng(4)              # targets: a stream of their own, the pools stay those of rng
     out = open(args.out, "a") if args.out else None
+
+    def emit(line):
+        print(json.dumps(line), flush=True)
+        if out:
+            out.write(json.dumps(line) + "\n")
+            out.flush()
     for pool_arg in args.pools.split(","):
         C = news.news_num - 1 if pool_arg == "all" else int(pool_arg)
         pool_news = (np.arange(1, news.news_num) if pool_arg == "all"
@@ -145,10 +159,32 @@ def main():
                             fallback_units_batch_caller=fb["caller"], units_per_user=int(plan.units(engine.TC_TRIPLES - 2)[0].numel()),
                             units_per_user_caller_order=int(caller.templates[engine.TC_TRIPLES - 2][0].numel()),
                             cache_news=news.news_num - 1, history=int(imp.hist_news.shape[1]), **info)
-                print(json.dumps(line), flush=True)
-                if out:
-                    out.write(json.dumps(line) + "\n")
-                    out.flush()
+                emit(line)
+
+            cutoffs = (10, 50, 100)
+            tgt = torch.from_numpy(pool_news[trng.integers(0, C, (args.users, args.targets))]).cuda()
+            tmask = torch.ones(tgt.shape, dtype=torch.bool, device="cuda")
+            pos = plan.positions(cache.news_num)[tgt[:ub].long()].contiguous()
+            rank = lambda: ops.pool_rank_metrics(s2, plan.index, pos, cutoffs, plan.news, None, hb[0], hb[1])
+            rank()
+            rank_ms = timed(rank, args.reps, 20)
+            ev = lambda: recommend.evaluate(model, cache, plan, *hist, tgt, tmask, cutoffs=cutoffs)
+            tk = lambda: recommend.top_k(model, cache, plan, *hist, 10)
+            ev(), tk()                                                                            # warm-up
+            te, tt = [], []
+            for _ in range(max(1, args.reps // 2)):                                               # alternated
+                te.append(timed(ev, 1))
+                tt.append(timed(tk, 1))
+            res = ev()
+            score_ms = float(np.median(t["sorted"]))
+            emit(dict(kind="evaluate", pool=C, users=args.users, targets=args.targets, cutoffs=list(cutoffs), users_per_launch=ub,
+                      score_ms_per_launch=round(score_ms, 3), rank_ms_per_launch=round(rank_ms, 4),
+                      rank_share_of_scoring=round(rank_ms / score_ms, 5),
+                      eval_users_per_s=round(args.users / (float(np.median(te)) / 1e3), 1),
+                      topk_users_per_s=round(args.users / (float(np.median(tt)) / 1e3), 1),
+                      eval_e2e_ms=round(float(np.median(te)), 2), topk_e2e_ms=round(float(np.median(tt)), 2),
+                      ranked_per_user=round(float(res.ranked.double().mean()), 3), fallback_units=res.fallback_units,
+                      cache_news=news.news_num - 1, history=int(imp.hist_news.shape[1]), **info))
     if out:
         out.close()
 
