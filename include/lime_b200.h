@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define LIME_B200_ABI_VERSION 6
+#define LIME_B200_ABI_VERSION 7
 
 /* Compile-time model geometry of the LIME-CROWN-CROWN configuration (config.py:54-91 defaults). */
 #define LIME_D        400   /* lime_output_dim == news_embedding_dim == attention_dim          */
@@ -318,6 +318,20 @@ int     lime_topic_pair_table(const float *topics, int64_t ldt, const float *tq,
  * (scale * x = hi + lo to 2^-22; the scoring kernel expects scale = LIME_CAND16_SCALE).  absmax (may be NULL): absmax[row * ldo] = max |x| of the row (inf for NaN). */
 int     lime_split_f16_pairs(const float *src, int64_t lds, int64_t rows, int32_t blocks, float scale, void *dst,
                              float *absmax, int64_t ldo, void *stream);
+/* Write n freshly built cache rows into a news-vector cache of news_num rows (csrc/cache.cu): source row r = hist [n,
+ * LIME_HIST_LD] and cand [n, LIME_CAND_LD] (contiguous, topic ids stamped) goes to destination row dst_rows[r] (int64) of
+ * every role, in one pass:
+ *   hist_rows [news_num, LIME_HIST_LD] and cand_rows [news_num, LIME_CAND_LD]: copies, max |cand[:, :1200]| (inf for NaN)
+ *     stamped into LIME_CAND_ABSMAX;
+ *   cand16 [>= news_num, LIME_CAND16_LD] fp16: the hi / lo pairs of lime_split_f16_pairs (scale LIME_CAND16_SCALE, same
+ *     arithmetic, bit for bit); the tail of bucket-pair rows after news_num is not touched;
+ *   news_meta [news_num, LIME_META_LD]: topic id | gw absmax | w absmax | B1 B2 B3 cb | 0;
+ *   hist_vg [news_num, 2*LIME_D]: vc and gw interleaved by 4 dims.
+ * The source rows may be the destination rows themselves (dst_rows[r] = r, same memory); otherwise they must not overlap the
+ * destination, and dst_rows must not repeat a row (the caller checks).  A destination outside [0, news_num) is skipped: the
+ * ids live on the device, so they are not checked here.  Every array 16-byte aligned.  n == 0: no launch. */
+int     lime_cache_write_rows(const float *hist, const float *cand, int64_t n, const int64_t *dst_rows, float *hist_rows,
+                              float *cand_rows, void *cand16, float *news_meta, float *hist_vg, int64_t news_num, void *stream);
 /* Diagnostic: per-phase clock64() totals of the tensor-core scoring kernel since the last call (thread 0 of every CTA;
  * slots listed in score_tc.cu), host buffer of 16 uint64.  Synchronises the device. */
 int     lime_score_phase_clocks(uint64_t *out16);

@@ -11,9 +11,9 @@ from . import news_modules as newsEncoders
 from . import user_modules as userEncoders
 from . import engine, ops, recommend, synth, trainer, training, util
 from .model import Model
-from .util import (NewsVectorCache, build_news_cache, compute_scores, evaluate_impressions,
-                   score_impressions)
+from .util import (NewsVectorCache, build_news_cache, compute_scores, evaluate_impressions, extend_news_cache,
+                   refresh_news_cache, score_impressions)
 
 __all__ = ["Model", "newsEncoders", "userEncoders", "layers", "util", "engine", "ops", "recommend", "synth", "trainer", "training",
-           "NewsVectorCache", "build_news_cache", "compute_scores", "evaluate_impressions",
-           "score_impressions"]
+           "NewsVectorCache", "build_news_cache", "compute_scores", "evaluate_impressions", "extend_news_cache",
+           "refresh_news_cache", "score_impressions"]

@@ -79,6 +79,7 @@ PROTOTYPES = {
     "lime_score_impressions_long": (C.c_int, [C.POINTER(LimeNewsCache), C.POINTER(LimeImpressions), C.POINTER(LimeImpressions), I32, I64,
                                               I32, I64, I32, I64, I32, P, P, P, P]),
     "lime_split_f16_pairs": (C.c_int, [P, I64, I64, I32, F32, P, P, I64, P]),
+    "lime_cache_write_rows": (C.c_int, [P, P, I64, P, P, P, P, P, P, I64, P]),
     "lime_score_phase_clocks": (C.c_int, [P]),
     "lime_score_smem_bytes": (I64, [I32, I32]),
     "lime_score_configure": (C.c_int, [I32, F32]),
@@ -127,7 +128,7 @@ PROTOTYPES = {
     "lime_click_score_bwd": (C.c_int, [P, P, P, P, I64, P, P, P]),
 }
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 _lib = None
 
 

@@ -297,21 +297,29 @@ class ScoringEngine:
         self._topic_table_n = 0
         self._topic_absmax = 0.0
 
-    def _register_topics(self, category, subCategory, hist, cand):
+    def _register_topics(self, category, subCategory, hist, cand, host_topics=None):
         """Assign compact topic ids to the news of freshly built cache rows and stamp them into the
-        rows (index building: torch plumbing; the logit table itself comes from lime_topic_pair_table)."""
-        key = category.long() * 1000003 + subCategory.long()
-        uniq, inverse = torch.unique(key, return_inverse=True)
-        first = torch.full((uniq.numel(),), key.numel(), dtype=torch.long, device=key.device)
-        first.scatter_reduce_(0, inverse, torch.arange(key.numel(), device=key.device), reduce="amin")
+        rows (index building: torch plumbing; the logit table itself comes from lime_topic_pair_table).
+        ``host_topics``: the same (category, subCategory) as numpy arrays, so the distinct keys are found on
+        the host instead of being read back from the device (same ids: keys ascending, first row of each)."""
+        if host_topics is not None:
+            hkey = np.asarray(host_topics[0], np.int64) * 1000003 + np.asarray(host_topics[1], np.int64)
+            uniq, first, inverse = np.unique(hkey, return_index=True, return_inverse=True)
+            uniq, first, inverse = uniq.tolist(), first.tolist(), torch.from_numpy(inverse.reshape(-1)).to(hist.device)
+        else:
+            key = category.long() * 1000003 + subCategory.long()
+            uniq, inverse = torch.unique(key, return_inverse=True)
+            first = torch.full((uniq.numel(),), key.numel(), dtype=torch.long, device=key.device)
+            first.scatter_reduce_(0, inverse, torch.arange(key.numel(), device=key.device), reduce="amin")
+            uniq, first = uniq.tolist(), first.tolist()
         lut = []
-        for k, r in zip(uniq.tolist(), first.tolist()):
+        for k, r in zip(uniq, first):
             if k not in self._topic_ids:
                 self._topic_ids[k] = len(self._topic_ids)
                 self._topic_vec.append(hist[r, HIST_T:HIST_T + TOPIC_LD].clone())
                 self._topic_tq.append(cand[r, CAND_TQ:CAND_TQ + TOPIC * HEADS + HEADS].clone())
             lut.append(self._topic_ids[k])
-        ids = torch.tensor(lut, dtype=torch.int32, device=key.device)[inverse]
+        ids = torch.tensor(lut, dtype=torch.int32, device=hist.device)[inverse]
         hist[:, HIST_TOPIC_ID].view(torch.int32).copy_(ids)
         cand[:, CAND_TOPIC_ID].view(torch.int32).copy_(ids)
 
@@ -431,15 +439,21 @@ class ScoringEngine:
         return F
 
     # -- per-news cache ----------------------------------------------------------------------------
-    def build_rows(self, title_text, body_text, category, subCategory, chunk=2048):
+    def build_rows(self, title_text, body_text, category, subCategory, chunk=2048, out=None, host_topics=None):
         """Encode news and derive both cache roles.  int32 device tensors [n,32], [n,128], [n], [n]
-        -> (hist_rows [n,852], cand_rows [n,1720])."""
+        -> (hist_rows [n,852], cand_rows [n,1720]).  ``out``: (hist, cand) contiguous views to write the rows
+        into; ``host_topics``: see _register_topics."""
         F = self.fold()
         lime = self.model.news_encoder
         n = title_text.shape[0]
         dev = title_text.device
-        hist = torch.zeros(n, HIST_LD, dtype=torch.float32, device=dev)
-        cand = torch.zeros(n, CAND_LD, dtype=torch.float32, device=dev)
+        if out is None:
+            hist = torch.zeros(n, HIST_LD, dtype=torch.float32, device=dev)
+            cand = torch.zeros(n, CAND_LD, dtype=torch.float32, device=dev)
+        else:
+            hist, cand = out
+            hist.zero_()
+            cand.zero_()
         Wc = self.news.prepare()["Wc"]
         for lo in range(0, n, chunk):
             hi = min(n, lo + chunk)
@@ -470,7 +484,7 @@ class ScoringEngine:
             ops.linear(h[:, HIST_T:HIST_T + TOPIC_LD], F["Atq"], F["atq0"],
                        out=c[:, CAND_TQ:CAND_TQ + TOPIC * HEADS + HEADS])           # tq, qb
         ops.row_absmax(hist[:, HIST_GW:HIST_GW + D], hist[:, HIST_GW_ABSMAX])
-        self._register_topics(category, subCategory, hist, cand)
+        self._register_topics(category, subCategory, hist, cand, host_topics)
         return hist, cand
 
     def _score_long(self, hist_rows, cand_rows, dimp, ch, prefix_main, tail_start, prefix_tail, pair_index_base, out, cand16, meta, hist_vg):

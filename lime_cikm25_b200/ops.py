@@ -507,6 +507,30 @@ def split_f16_pairs(src, blocks=3, absmax=None, scale=CAND16_SCALE, out=None):
     return dst
 
 
+def cache_write_rows(hist, cand, dst_rows, hist_rows, cand_rows, cand16, meta, hist_vg):
+    """lime_cache_write_rows: freshly built rows hist [n, 852] / cand [n, 1720] (ScoringEngine.build_rows) -> row
+    dst_rows[r] (int64 [n], distinct) of every role of a cache of news_num = hist_rows.shape[0] rows: hist_rows, cand_rows
+    (max |w| stamped into column 1207), cand16 [>= news_num, 2400] fp16 (what split_f16_pairs writes), meta [news_num, 8]
+    (ScoringEngine.news_meta) and hist_vg [news_num, 800] (engine.interleave_vg).  All contiguous.  The source may be the
+    destination rows themselves (dst_rows = 0..n-1 over the same memory)."""
+    lib = _lib.require_device()
+    n, news_num = int(hist.shape[0]), int(hist_rows.shape[0])
+    shapes = ((hist, (n, 852), torch.float32), (cand, (n, 1720), torch.float32), (dst_rows, (n,), torch.int64),
+              (hist_rows, (news_num, 852), torch.float32), (cand_rows, (news_num, 1720), torch.float32),
+              (meta, (news_num, 8), torch.float32), (hist_vg, (news_num, 800), torch.float32))
+    for t, shape, dtype in shapes:
+        if tuple(t.shape) != shape or t.dtype != dtype or not t.is_contiguous():
+            raise _lib.LimeError("cache_write_rows: expected a contiguous %s %s tensor, got %s %s"
+                                 % (dtype, list(shape), t.dtype, list(t.shape)))
+    if cand16.dtype != torch.float16 or not cand16.is_contiguous() or cand16.dim() != 2 or cand16.shape[1] != 2400 \
+            or cand16.shape[0] < news_num:
+        raise _lib.LimeError("cache_write_rows: cand16 must be a contiguous fp16 [>= news_num, 2400] tensor")
+    check(lib.lime_cache_write_rows(_ptr(hist, torch.float32, "hist"), _ptr(cand, torch.float32, "cand"), n,
+                                    _ptr(dst_rows, torch.int64, "dst_rows"), hist_rows.data_ptr(), cand_rows.data_ptr(),
+                                    _ptr(cand16, torch.float16, "cand16"), meta.data_ptr(), hist_vg.data_ptr(), news_num,
+                                    _stream()), "lime_cache_write_rows")
+
+
 SCORE_AUTO, SCORE_EXACT, SCORE_FORCE_FALLBACK = 0, 1, 2
 _score_mode = SCORE_AUTO
 
