@@ -179,34 +179,35 @@ def test_reference_model_py_over_plugin_classes(lib, golden_dir):
     assert rel(torch.cat(out).numpy(), g["scores"]) < TOL
 
 
-def _stage_b_oracle(model, sd, cfg, cache, news, imp, prefix):
-    """CPU oracle of the user encoder + click score on the GPU-built LIME vectors (isolates Stage B)."""
+def _stage_b_oracle(model, sd, cfg, cache, news, imp, prefix, dtype=torch.float32, remaining=None):
+    """CPU oracle of the user encoder + click score on the GPU-built LIME vectors (isolates Stage B):
+    O.score_from_vectors per impression.  ``prefix``: the GraphSAGE prefix, an int or one per pair [P];
+    ``remaining``: the pairs' remaining lifetime [P] (default: life - freshness in fp32, as the callers derive it)."""
     se = model.scoring
-    out = np.zeros(imp.num_pairs, np.float32)
-    H = imp.hist_news.shape[1]
+    out = np.zeros(imp.num_pairs, np.float64 if dtype == torch.float64 else np.float32)
+    pre = np.broadcast_to(np.asarray(prefix, np.int64), (imp.num_pairs,))
+    rem = imp.cand_life - imp.cand_fresh if remaining is None else np.asarray(remaining, np.float32)
     for i in range(imp.num_impressions):
+        p0, p1 = int(imp.cand_off[i]), int(imp.cand_off[i + 1])
+        if p1 == p0:
+            continue
         hn = torch.as_tensor(imp.hist_news[i]).long()
+        cn = torch.as_tensor(imp.cand_news[p0:p1]).long()
         hv = se.lime_vectors(cache.hist_rows[hn.to(DEV)], torch.as_tensor(imp.hist_fresh[i]).to(DEV),
                              torch.as_tensor(imp.hist_life[i]).to(DEV)).cpu()
-        for p in range(imp.cand_off[i], imp.cand_off[i + 1]):
-            cn = int(imp.cand_news[p])
-            cv = se.lime_vectors(cache.hist_rows[cn:cn + 1], torch.as_tensor(imp.cand_fresh[p:p + 1]).to(DEV),
-                                 torch.as_tensor(imp.cand_life[p:p + 1]).to(DEV)).cpu()
-            u = O.crown_user(sd, hv.view(1, H, -1), torch.as_tensor(news.category[hn]).view(1, H),
-                             torch.as_tensor(news.subCategory[hn]).view(1, H),
-                             torch.as_tensor(news.category[cn:cn + 1]).view(1, 1),
-                             torch.as_tensor(news.subCategory[cn:cn + 1]).view(1, 1),
-                             torch.as_tensor(imp.hist_mask[i]).view(1, H), cv.view(1, 1, -1), cfg,
-                             prefix_len=prefix)
-            r = torch.tensor(imp.cand_life[p] - imp.cand_fresh[p])
-            out[p] = float((u * cv.view(1, 1, -1)).sum() * O.lifetime_weight(r, cfg))
+        cv = se.lime_vectors(cache.hist_rows[cn.to(DEV)], torch.as_tensor(imp.cand_fresh[p0:p1]).to(DEV),
+                             torch.as_tensor(imp.cand_life[p0:p1]).to(DEV)).cpu()
+        hn_, cn_ = imp.hist_news[i], imp.cand_news[p0:p1]
+        out[p0:p1] = O.score_from_vectors(sd, cfg, hv, news.category[hn_], news.subCategory[hn_], imp.hist_mask[i], cv,
+                                          news.category[cn_], news.subCategory[cn_], rem[p0:p1], pre[p0:p1], dtype).numpy()
     return out
 
 
-@pytest.mark.parametrize("H,cand,prefix", [(200, 70, 32), (100, 5, 120), (20, 300, 7), (50, 1, 64)])
+@pytest.mark.parametrize("H,cand,prefix", [(200, 70, 32), (100, 5, 120), (20, 300, 7), (50, 1, 64), (223, 40, 100)])
 def test_scoring_kernel_sweep_shapes(lib, H, cand, prefix):
-    """Sweep shapes of BASELINE.json configs[4]: history up to 200 (multi-chunk register tiling),
-    300 candidates (multi-unit impressions), GraphSAGE prefix below / above H."""
+    """Sweep shapes of BASELINE.json configs[4]: history up to 223 (multi-chunk register tiling),
+    300 candidates (multi-unit impressions), GraphSAGE prefix below / above H.  The exact kernel and the
+    default mode (cache operands passed: tensor cores, chunked beyond 56 slots) against the fp64 reference."""
     cfg = make_config(vocabulary_size=400, batch_size=128, max_history_num=H, word_embedding_init="skip")
     model = L.Model(cfg)
     model.initialize()
@@ -220,8 +221,10 @@ def test_scoring_kernel_sweep_shapes(lib, H, cand, prefix):
         cache = util.build_news_cache(model, news)
         dimp = engine.DeviceImpressions(imp, DEV)
         got = model.scoring.score(cache.hist_rows, cache.cand_rows, dimp, prefix_main=prefix).cpu().numpy()
-        want = _stage_b_oracle(model, sd, cfg, cache, news, imp, prefix)
-    assert rel(got, want) < TOL
+        tc = model.scoring.score(cache.hist_rows, cache.cand_rows, dimp, prefix_main=prefix, cand16=cache.cand16, meta=cache.meta,
+                                 hist_vg=cache.hist_vg).cpu().numpy()
+        want = _stage_b_oracle(model, sd, cfg, cache, news, imp, prefix, torch.float64)
+    assert rel(got, want) < TOL and rel(tc, want) < TOL
 
 
 def test_bucket_sweep_and_flags(lib):
@@ -511,17 +514,19 @@ def test_tensor_core_scoring_paths(lib):
     assert np.isfinite(s_big.cpu().numpy()).all()
 
 
-@pytest.mark.parametrize("H,prefix", [(100, 32), (200, 32), (112, 130)])
+@pytest.mark.parametrize("H,prefix", [(100, 32), (200, 32), (112, 130), (200, 103), (224, 57), (64, 40)])
 def test_long_history_on_the_tensor_core_path(lib, H, prefix):
     """H > 56 (BASELINE.json configs[4]): the history is cut into chunks of <= 56 slots, the attention weights over the FULL
     history come from a pre-pass, every chunk runs on the tensor-core kernel and the partial pooling states are merged
-    (lime_score_impressions_long).  Same scores as the exact per-pair kernel, no unit handed to the fallback; ragged histories,
-    a masked tail, multi-unit impressions and a GraphSAGE prefix above H included."""
+    (lime_score_impressions_long).  Same scores as the exact per-pair kernel and as the fp64 reference, no unit handed to the
+    fallback; ragged histories, a masked tail, multi-unit impressions and GraphSAGE prefixes that end inside chunk 1
+    (H = 64, 224) or chunk 2 (H = 200, prefix 103), or lie above H, included."""
     from lime_cikm25_b200 import ops
     cfg = make_config(vocabulary_size=400, batch_size=128, max_history_num=H, word_embedding_init="skip")
     model = L.Model(cfg)
     model.initialize()
     synth.synthetic_parameters(model, 5)
+    sd = {k: v.detach().clone() for k, v in model.state_dict().items()}
     model = model.to(DEV).eval()
     news = synth.make_news_table(300, vocabulary_size=400, seed=H)
     imp = synth.make_impressions(40, news.news_num, max_history=H, cand_mean=30.0, near_zero_frac=0.3, seed=H + 1)
@@ -539,4 +544,6 @@ def test_long_history_on_the_tensor_core_path(lib, H, prefix):
                                        cand16=cache.cand16, meta=cache.meta, hist_vg=cache.hist_vg).cpu().numpy()
         finally:
             ops.score_configure(ops.SCORE_AUTO, 1e-6)
-    assert rel(got, want) < TOL
+        ref = _stage_b_oracle(model, sd, cfg, cache, news, imp, prefix, torch.float64)
+    assert rel(got, want) < 5e-5
+    assert rel(got, ref) < TOL and rel(want, ref) < TOL

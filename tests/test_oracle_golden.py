@@ -82,3 +82,28 @@ def test_oracle_ranks_and_metrics_match_reference(golden_dir):
     m, ranks = O.evaluate_impressions(s, y)
     assert np.array_equal(np.concatenate(ranks), g["ranks"])      # stable, -0.0 == 0.0
     assert np.allclose(m, g["metrics"], rtol=0, atol=1e-12)
+
+
+@pytest.mark.parametrize("case", ["small_bs8", "bs64"])
+def test_score_from_vectors_reproduces_model_forward(case, golden_dir):
+    """score_from_vectors (Stage B from LIME vectors, the fp64 reference of the scoring kernels) is model_forward's own
+    user encoder + click score: fed model_forward's cand / hist parts, it gives the same logits, with the GraphSAGE
+    prefix of the reference's mini-batch (the runtime batch size, shorter on the last batch).  In fp32 the two differ
+    only by the batching of the same products (the oracle's own fp32-vs-fp32 bar); in fp64 they agree to rounding."""
+    spec, cfg, news, imp, g, sd = load_case(case, golden_dir)
+    for dtype, bar in ((torch.float32, 1e-5), (torch.float64, 1e-12)):
+        got, want = [], []
+        with torch.no_grad():
+            for batch in synth.impressions_to_pair_batches(news, imp, cfg.batch_size):
+                logits, parts = O.model_forward(sd, batch, cfg, dtype, return_parts=True)
+                u_cat, u_sub, u_mask, n_cat, n_sub = (torch.as_tensor(np.asarray(batch[k])) for k in (1, 2, 11, 15, 16))
+                B = logits.shape[0]
+                for b in range(B):
+                    got.append(O.score_from_vectors(sd, cfg, parts["hist"][b], u_cat[b], u_sub[b], u_mask[b], parts["cand"][b],
+                                                    n_cat[b].view(1), n_sub[b].view(1), parts["remaining"][b].view(1), B, dtype))
+                want.append(logits.view(-1))
+        got, want = torch.cat(got).numpy(), torch.cat(want).numpy()
+        assert got.dtype == want.dtype == {torch.float32: np.float32, torch.float64: np.float64}[dtype]
+        assert np.array_equal(got == 0, want == 0)
+        assert rel(got, want) < bar, (dtype, rel(got, want))
+    assert rel(got, g["scores"]) < 1e-4            # fp64 against the reference's fp32 run: its own rounding only
