@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define LIME_B200_ABI_VERSION 7
+#define LIME_B200_ABI_VERSION 8
 
 /* Compile-time model geometry of the LIME-CROWN-CROWN configuration (config.py:54-91 defaults). */
 #define LIME_D        400   /* lime_output_dim == news_embedding_dim == attention_dim          */
@@ -306,6 +306,25 @@ int lime_score_impressions(const LimeNewsCache *cache, const LimeImpressions *im
                            int32_t prefix_tail, float *scores, int32_t *scratch,
                            void *stream);
 int     lime_score_configure(int32_t mode, float tolerance);
+/* Explain scored pairs: the exact kernel's per-slot terms of every (impression, candidate) pair, for the few pairs a user
+ * is shown.  Replaces, per pair, the same reference lines as lime_score_impressions
+ *   CandidateAware_ClickedNewsAttention.forward   layers.py:52-93
+ *   userEncoders.CROWN.forward tail               userEncoders.py:121,151-171
+ *   RemainingLifetimeWeighting.forward            util.py:23-49
+ * and writes the score as a sum of one term per history slot plus a bias (DESIGN.md "Explaining a recommendation"):
+ *   scores[p]                   the score, the same expression (and, in SCORE_EXACT mode, the same bits) as
+ *                               lime_score_impressions;
+ *   weight[p]                   w = the remaining-lifetime weight;
+ *   bias[p]                     w * (b_l . c + (1/P) sum_{j < P - H} user_node_j . W_l^T c), the part no history slot carries;
+ *   alpha[p * H + h]            the candidate-query pooling weight of slot h (userEncoders.py:164, unmasked);
+ *   topic_attn[p * H + h]       the candidate-aware weight of slot h (layers.py:81, unmasked);
+ *   contrib[p * H + h]          w * (alpha_h x_h . W_r^T c + [h < min(P, H)] x_h . W_l^T c / P),
+ * so scores[p] = bias[p] + sum_h contrib[p * H + h] up to fp32 rounding.  P = prefix_main for every pair.  Always runs the
+ * exact kernel, whatever lime_score_configure selected.  A unit with unit_count 0 is skipped; the pairs no unit covers are
+ * not written.  H in [1, 224], prefix_main in [1, H + user_nodes], every pointer non-null; scratch: lime_score_scratch_ints. */
+int     lime_explain_pairs(const LimeNewsCache *cache, const LimeImpressions *imp, int32_t prefix_main, float *scores,
+                           float *alpha, float *topic_attn, float *contrib, float *bias, float *weight, int32_t *scratch,
+                           void *stream);
 /* Candidate-aware attention logits depend on the news only through their (category, subCategory)
  * pair (layers.py:66-70 on the 50-d topic representations), so they are tabulated once per checkpoint:
  *   out[(tc * T + th) * LIME_TOPIC_TAB_LD + head] = exp(Q_head(topic tc) . K_head(topic th) / sqrt(D))   (softmax numerators)

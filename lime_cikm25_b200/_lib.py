@@ -83,6 +83,7 @@ PROTOTYPES = {
     "lime_score_phase_clocks": (C.c_int, [P]),
     "lime_score_smem_bytes": (I64, [I32, I32]),
     "lime_score_configure": (C.c_int, [I32, F32]),
+    "lime_explain_pairs": (C.c_int, [C.POINTER(LimeNewsCache), C.POINTER(LimeImpressions), I32, P, P, P, P, P, P, P, P]),
     "lime_score_scratch_ints": (I64, [I32]),
     "lime_score_tile_c": (I32, [I32]),
     "lime_sizeof_news_cache": (I64, []),
@@ -128,7 +129,7 @@ PROTOTYPES = {
     "lime_click_score_bwd": (C.c_int, [P, P, P, P, I64, P, P, P]),
 }
 
-ABI_VERSION = 7
+ABI_VERSION = 8
 _lib = None
 
 

@@ -128,8 +128,20 @@ __host__ __device__ inline size_t smem_carve(SmemLayout *L, unsigned char *base,
     return off;
 }
 
-template <int MAXP>
-__global__ void __launch_bounds__(kThreads, 1) score_kernel(const ScoreArgs args) {
+// Per-pair terms of the score for lime_explain_pairs: [pair][H] rows for alpha / topic_attn / contrib, [pair] for
+// bias / weight.  Unused (all NULL) by the scoring instantiations.
+struct ExplainOut {
+    float *alpha;
+    float *topic_attn;
+    float *contrib;
+    float *bias;
+    float *weight;
+};
+
+// kExplain: phase 3 also writes the decomposition score = bias + sum_h contrib[h] (lime_explain_pairs); the score
+// itself is the same expression in both instantiations.
+template <int MAXP, bool kExplain>
+__global__ void __launch_bounds__(kThreads, 1) score_kernel(const ScoreArgs args, const ExplainOut ex) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const LimeNewsCache &C = args.cache;
     const LimeImpressions &I = args.imp;
@@ -162,6 +174,9 @@ __global__ void __launch_bounds__(kThreads, 1) score_kernel(const ScoreArgs args
         const int imp = I.unit_imp[unit];
         const int pair0 = I.unit_pair0[unit];
         const int cnt = I.unit_count[unit];
+        if constexpr (kExplain) {
+            if (cnt <= 0) continue;   // a user whose explained news are all padding
+        }
 
         // ---------------- phase 0: unit metadata + topic tile -----------------------------------
         for (int h = tid; h < H; h += kThreads) {
@@ -490,6 +505,22 @@ __global__ void __launch_bounds__(kThreads, 1) score_kernel(const ScoreArgs args
                 const float base = (ms + un) / (float)P + S.cscal[c * 8 + 6] + acc / l;
                 args.scores[(long long)pair0 + c] = base * S.cw[c];
             }
+            if constexpr (kExplain) {
+                // contrib_h = w (alpha_h y_h + [h < min(P, H)] z_h / P), bias = w (un / P + b_l . c)
+                const long long pair = (long long)pair0 + c;
+                const float w = S.cw[c];
+                if (lane == 0) {
+                    ex.bias[pair] = w * (un / (float)P + S.cscal[c * 8 + 6]);
+                    ex.weight[pair] = w;
+                }
+                for (int hh = lane; hh < H; hh += 32) {
+                    const float al = __expf(S.lg_s[c * H + hh] - m) / l;
+                    const float zp = hh < pz ? S.z_s[c * H + hh] / (float)P : 0.0f;
+                    ex.alpha[pair * H + hh] = al;
+                    ex.topic_attn[pair * H + hh] = S.a_s[c * H + hh];
+                    ex.contrib[pair * H + hh] = w * fmaf(al, S.y_s[c * H + hh], zp);
+                }
+            }
         }
     }
 }
@@ -500,8 +531,8 @@ namespace lime {
 
 int64_t score_exact_smem(int H, int TC) { return (int64_t)smem_carve(nullptr, nullptr, H, TC); }
 
-// exact kernel over all units (unit_list == NULL) or over the device-side fallback list
-int launch_score_exact(const ScoreArgs &a, int grid_limit, cudaStream_t st) {
+template <bool kExplain>
+static int launch_exact(const ScoreArgs &a, const ExplainOut &ex, int grid_limit, cudaStream_t st) {
     const int H = a.imp.max_history, TC = a.imp.tile_c;
     const size_t smem = smem_carve(nullptr, nullptr, H, TC);
     LIME_CHECK_ARG(smem <= 232448, "lime_score_impressions: (H=%d, tile_c=%d) needs %zu B of shared memory", H, TC, smem);
@@ -510,17 +541,22 @@ int launch_score_exact(const ScoreArgs &a, int grid_limit, cudaStream_t st) {
     if (grid > grid_limit) grid = grid_limit;
     const int passes = (H + 31) / 32;
     if (passes <= 2) {
-        LIME_CUDA(cudaFuncSetAttribute(score_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        score_kernel<2><<<grid, kThreads, smem, st>>>(a);
+        LIME_CUDA(cudaFuncSetAttribute(score_kernel<2, kExplain>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        score_kernel<2, kExplain><<<grid, kThreads, smem, st>>>(a, ex);
     } else if (passes <= 4) {
-        LIME_CUDA(cudaFuncSetAttribute(score_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        score_kernel<4><<<grid, kThreads, smem, st>>>(a);
+        LIME_CUDA(cudaFuncSetAttribute(score_kernel<4, kExplain>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        score_kernel<4, kExplain><<<grid, kThreads, smem, st>>>(a, ex);
     } else {
-        LIME_CUDA(cudaFuncSetAttribute(score_kernel<7>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        score_kernel<7><<<grid, kThreads, smem, st>>>(a);
+        LIME_CUDA(cudaFuncSetAttribute(score_kernel<7, kExplain>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        score_kernel<7, kExplain><<<grid, kThreads, smem, st>>>(a, ex);
     }
     LIME_LAUNCH_CHECK("score_kernel");
     return 0;
+}
+
+// exact kernel over all units (unit_list == NULL) or over the device-side fallback list
+int launch_score_exact(const ScoreArgs &a, int grid_limit, cudaStream_t st) {
+    return launch_exact<false>(a, ExplainOut{}, grid_limit, st);
 }
 
 // process-wide scoring mode (lime_score_configure)
@@ -599,6 +635,33 @@ extern "C" int lime_score_impressions(const LimeNewsCache *cache, const LimeImpr
     a.unit_list = scratch + 4;
     a.unit_list_count = scratch + 1;
     return launch_score_exact(a, imp->num_units, st);
+}
+
+extern "C" int lime_explain_pairs(const LimeNewsCache *cache, const LimeImpressions *imp, int32_t prefix_main, float *scores,
+                                  float *alpha, float *topic_attn, float *contrib, float *bias, float *weight, int32_t *scratch,
+                                  void *stream) {
+    LIME_CHECK_ARG(cache && imp && scores && alpha && topic_attn && contrib && bias && weight && scratch,
+                   "lime_explain_pairs: null argument");
+    const int H = imp->max_history, TC = imp->tile_c;
+    LIME_CHECK_ARG(H >= 1 && H <= 224, "lime_explain_pairs: max_history %d not in [1,224]", H);
+    LIME_CHECK_ARG(TC >= 1, "lime_explain_pairs: tile_c %d < 1", TC);
+    LIME_CHECK_ARG(cache->num_buckets >= 1 && cache->news_num >= 1, "lime_explain_pairs: empty cache");
+    LIME_CHECK_ARG(prefix_main >= 1 && prefix_main <= H + cache->user_nodes,
+                   "lime_explain_pairs: prefix_main %d not in [1, %d]", prefix_main, H + cache->user_nodes);
+    if (imp->num_units <= 0) return 0;
+
+    ScoreArgs a = {};
+    a.cache = *cache;
+    a.imp = *imp;
+    a.tail_start = 1LL << 62;
+    a.prefix_main = prefix_main;
+    a.prefix_tail = prefix_main;
+    a.bucket_scale = (float)((double)cache->num_buckets / 7.0);
+    a.ln_eps = 1e-5f;
+    a.scores = scores;
+    a.work_counter = scratch;
+    const ExplainOut ex = {alpha, topic_attn, contrib, bias, weight};
+    return launch_exact<true>(a, ex, imp->num_units, as_stream(stream));
 }
 
 // ---- histories longer than the tensor-core kernel's 56 slots (BASELINE.json configs[4]: history 100 / 200) ------------------

@@ -746,6 +746,43 @@ class DeviceImpressions:
         return self
 
     @classmethod
+    def from_lists(cls, plan, news_num, news, hist_news, hist_mask, hist_fresh, hist_life):
+        """Each of Ub users (histories [Ub, H], device tensors) against its own k news: row u of ``news`` [Ub, k] (cache rows
+        of ``plan``'s pool, -1 = padding), freshness / lifetime / remaining lifetime gathered from the plan through
+        plan.positions(news_num).  Impression u = user u.  Padding is not scored: every row's news are moved to its front
+        in their order, so pair u * k + j is the j-th non-padding news of row u, and ``order`` [Ub, k] (int64) is the column
+        of ``news`` pair u * k + j came from.  Units are runs of at most tile_c of them; a unit past a row's last news has
+        no candidates (lime_explain_pairs skips it).  Device tensors only, no host copies."""
+        self = cls.__new__(cls)
+        dev = hist_mask.device
+        Ub, H = hist_mask.shape
+        k = news.shape[1]
+        if Ub * k >= 2 ** 31:
+            raise _lib.LimeError("from_lists: %d users x %d news exceed the int32 pair index" % (Ub, k))
+        i32 = dict(dtype=torch.int32, device=dev)
+        self.tile_c = choose_tile_c(H)
+        self.order = torch.sort((news < 0).to(torch.uint8), dim=1, stable=True).indices
+        cand = news.gather(1, self.order)
+        pos = plan.positions(news_num)[cand.clamp_min(0)].long().clamp_min(0).reshape(-1)
+        nu = (k + self.tile_c - 1) // self.tile_c
+        self.max_history, self.num_pairs, self.num_impressions, self.num_units = H, Ub * k, Ub, Ub * nu
+        self.device = dev
+        self.planned_buckets = None
+        u = torch.arange(Ub, **i32).view(Ub, 1)
+        j0 = torch.arange(0, nu * self.tile_c, self.tile_c, **i32).view(1, nu)
+        valid = (cand >= 0).sum(dim=1, dtype=torch.int32).view(Ub, 1)
+        self.dev = dict(
+            hist_news=hist_news.to(torch.int32).contiguous(), hist_mask=hist_mask.to(torch.uint8).contiguous(),
+            hist_fresh=hist_fresh.float().contiguous(), hist_life=hist_life.float().contiguous(),
+            cand_news=cand.to(torch.int32).reshape(-1), cand_fresh=plan.fresh[pos], cand_life=plan.life[pos],
+            unit_imp=u.expand(Ub, nu).reshape(-1), unit_pair0=(u * k + j0).reshape(-1),
+            unit_count=(valid - j0).clamp(0, self.tile_c).reshape(-1))
+        if plan.remaining is not None:
+            self.dev["cand_remaining"] = plan.remaining[pos]
+        self.work_counter = torch.zeros(int(_lib.load().lime_score_scratch_ints(self.num_units)), **i32)
+        return self
+
+    @classmethod
     def from_pairs(cls, hist_mask, hist_fresh, hist_life, cand_fresh, cand_life, cand_remaining, n_cand):
         """Per-pair layout of Model.forward (one impression per sample, ``n_cand`` candidates each):
         the freshly encoded batch is its own news cache with history rows first

@@ -547,6 +547,29 @@ def score_mode():
     return _score_mode
 
 
+EXPLAIN_MAX_HISTORY = 224      # lime_explain_pairs: H in [1, 224]
+
+
+def explain_pairs(cache, imp, prefix_main, scores, alpha, topic_attn, contrib, bias, weight, scratch):
+    """lime_explain_pairs: the exact scoring kernel over the LimeNewsCache / LimeImpressions structs ``cache`` / ``imp``
+    (every pair's GraphSAGE prefix ``prefix_main``), writing per pair p the score, bias and lifetime weight (scores / bias /
+    weight [P] fp32) and per history slot h the pooling weight, candidate-aware weight and contribution (alpha / topic_attn /
+    contrib [P, H] fp32), score = bias + sum_h contrib up to rounding.  Pairs no unit covers are not written.  scratch:
+    int32 [>= lime_score_scratch_ints(num_units)].  All contiguous CUDA tensors; runs the exact kernel in every scoring mode."""
+    lib = _lib.require_device()
+    P, H = int(scores.numel()), int(imp.max_history)
+    for t, shape, name in ((scores, (P,), "scores"), (bias, (P,), "bias"), (weight, (P,), "weight"), (alpha, (P, H), "alpha"),
+                           (topic_attn, (P, H), "topic_attn"), (contrib, (P, H), "contrib")):
+        if tuple(t.shape) != shape or not t.is_contiguous():
+            raise ValueError("explain_pairs: %s must be a contiguous %s tensor, got %s" % (name, list(shape), list(t.shape)))
+    if scratch.numel() < int(lib.lime_score_scratch_ints(imp.num_units)) or not scratch.is_contiguous():
+        raise ValueError("explain_pairs: scratch must hold lime_score_scratch_ints(num_units) int32")
+    f = lambda t, name: _ptr(t, torch.float32, name)
+    check(lib.lime_explain_pairs(ctypes.byref(cache), ctypes.byref(imp), int(prefix_main), f(scores, "scores"), f(alpha, "alpha"),
+                                 f(topic_attn, "topic_attn"), f(contrib, "contrib"), f(bias, "bias"), f(weight, "weight"),
+                                 _ptr(scratch, torch.int32, "scratch"), _stream()), "lime_explain_pairs")
+
+
 # ---- training kernels (csrc/train_kernels.cu) -------------------------------------------------------
 def gemm(a, a_kmajor, b, b_kmajor, m, n, k, out=None, alpha=1.0, accumulate=False, bf16=False):
     """out[m, n] (+)= alpha * op(a) @ op(b) (lime_gemm / lime_gemm_bf16; see include/lime_b200.h for the layouts)."""

@@ -21,6 +21,16 @@ Offline evaluation of the same lists: hold out each user's later clicks and rank
 A target's rank counts every position top_k could return to the user (other targets included), in top_k's order, so
 rank r <= k means top_k(k) returns that news at position r.  lime_pool_rank_metrics ranks them on the device.
 
+Why a news item was recommended: the score of every (user, news) pair split into one term per history slot.
+
+    ex = recommend.explain(model, cache, plan, hist_news, hist_mask, hist_fresh, hist_life, news)   # news [U, k], e.g. res.news
+    ex.score / ex.weight / ex.bias [U, k] fp32, ex.contrib / ex.alpha / ex.topic_attention [U, k, H] fp32,
+    ex.top_history(m) -> [U, k, m] int64 history slots, largest contribution first
+
+score = bias + sum_h contrib[h]: contrib[h] = w (alpha_h x_h . W_r^T c + [h < min(P, H)] x_h . W_l^T c / P), bias = w (b_l . c +
+the user-node rows' share of the GraphSAGE mean), w the remaining-lifetime weight (DESIGN.md "Explaining a recommendation").
+lime_explain_pairs computes the terms on the exact scoring kernel.
+
 GraphSAGE semantics: every (user, news) pair is scored as it would be in a FULL mini-batch of config.batch_size of the
 reference's eval loop (SURVEY.md section 8a row 10: the user-node prefix length follows the runtime batch size), so a
 score depends on neither the pool's size or order nor on how users are batched.
@@ -35,6 +45,7 @@ from .engine import HIST_TOPIC_ID, TC_TRIPLES, DeviceImpressions, PoolPlan, _hos
 from .util import remaining_lifetime
 
 PAIR_BUDGET = 1 << 24        # (user, news) pairs per scoring launch: 64 MB of scores, far from the int32 pair index
+EXPLAIN_BUDGET = 1 << 24     # floats of per-batch explain output (3 H + 3 per pair): 64 MB of scratch
 
 
 def _host(a, dtype):
@@ -219,3 +230,81 @@ def evaluate(model, cache, plan, hist_news, hist_mask, hist_fresh, hist_life, ta
             for dst, src in zip((ev.rank, ev.ranked, ev.eligible, ev.metrics), r):
                 dst[u0:u1] = src
     return ev
+
+
+class Explanation:
+    """Result of explain (device tensors; see the module docstring).  Padded pairs hold NaN everywhere."""
+
+    def __init__(self, score, weight, bias, contrib, alpha, topic_attention, hist_mask):
+        self.score, self.weight, self.bias = score, weight, bias
+        self.contrib, self.alpha, self.topic_attention = contrib, alpha, topic_attention
+        self.hist_mask = hist_mask
+
+    def top_history(self, m):
+        """[U, k, m] int64: the history slots of every pair's m largest contributions, largest first, equal contributions by
+        ascending slot.  Only masked-in slots are returned (masked-out slots keep their contributions in ``contrib``: the
+        unmasked softmaxes of the reference give them weight, but they are not clicks); -1 pads rows with fewer masked-in
+        slots than m, and every slot of a padded pair."""
+        if not isinstance(m, (int, np.integer)) or m < 1:
+            raise ValueError("m must be an integer >= 1")
+        U, k, H = self.contrib.shape
+        ok = self.hist_mask.bool().view(U, 1, H).expand(U, k, H) & ~torch.isnan(self.score).view(U, k, 1)
+        order = torch.sort(self.contrib, dim=-1, descending=True, stable=True).indices
+        order = order.gather(-1, torch.sort((~ok.gather(-1, order)).to(torch.uint8), dim=-1, stable=True).indices)
+        n = min(int(m), H)
+        top = torch.where(ok.gather(-1, order[..., :n]), order[..., :n], -1)
+        if n < m:
+            top = torch.cat([top, top.new_full((U, k, m - n), -1)], dim=-1)
+        return top
+
+
+def explain(model, cache, plan, hist_news, hist_mask, hist_fresh, hist_life, news):
+    """Explain the scores of U users' lists: histories as in top_k (H <= 224), news [U, k] cache rows of ``plan``'s pool or
+    -1 (padding, as in TopK.news).  Every pair is scored exactly as top_k scores it (the plan's freshness, lifetime and
+    remaining lifetime, a full mini-batch GraphSAGE prefix), on the exact kernel in every scoring mode: the score equals
+    top_k's bit for bit under ops.SCORE_EXACT and to the tensor-core tolerance otherwise.  -> Explanation.
+    Masked-out history slots keep their real contributions in ``contrib`` (the reference's pooling and second
+    candidate-aware softmax are unmasked, so the model gives them weight); top_history never returns them.
+    Raises ValueError before any launch for mismatched shapes, H outside [1, 224], and news that are out of range or not
+    in the pool; that check reads the device once.  Users are explained in batches of EXPLAIN_BUDGET / (k (3 H + 3))."""
+    dev = plan.device
+    hist = _histories(plan, hist_news, hist_mask, hist_fresh, hist_life)
+    hn, hm = hist[0], hist[1]
+    U, H = hn.shape
+    if not 1 <= H <= ops.EXPLAIN_MAX_HISTORY:
+        raise ValueError("max_history must lie in [1, %d]" % ops.EXPLAIN_MAX_HISTORY)
+    nw = (news if torch.is_tensor(news) else torch.from_numpy(np.asarray(news))).to(dev, torch.int64)
+    if nw.dim() != 2 or nw.shape[0] != U or nw.shape[1] < 1:
+        raise ValueError("news must be a [users, k] array with k >= 1, one row per history")
+    n = cache.news_num
+    pos = plan.positions(n)
+    bad = (nw != -1) & ((nw < 0) | (nw >= n) | (pos[nw.clamp(0, n - 1)] < 0))
+    if bool(bad.any()):                                        # the one device read
+        raise ValueError("news must be -1 or cache rows of the plan's pool")
+    k = nw.shape[1]
+    f32 = dict(dtype=torch.float32, device=dev)
+    nan = float("nan")
+    ex = Explanation(torch.full((U, k), nan, **f32), torch.full((U, k), nan, **f32), torch.full((U, k), nan, **f32),
+                     torch.full((U, k, H), nan, **f32), torch.full((U, k, H), nan, **f32), torch.full((U, k, H), nan, **f32),
+                     hm)
+    ub = max(1, min(U, EXPLAIN_BUDGET // (k * (3 * H + 3))))
+    vec = torch.empty(3, ub * k, **f32)                        # score, weight, bias in the compacted pair order
+    mat = torch.empty(3, ub * k, H, **f32)                     # contrib, alpha, topic attention
+    cs = model.scoring.cache_struct(cache.hist_rows, cache.cand_rows)
+    with torch.no_grad():
+        for u0 in range(0, U, ub):
+            u1 = min(U, u0 + ub)
+            b = u1 - u0
+            dimp = DeviceImpressions.from_lists(plan, n, nw[u0:u1], hn[u0:u1], hm[u0:u1], hist[2][u0:u1], hist[3][u0:u1])
+            v, mt = vec[:, :b * k], mat[:, :b * k]
+            v.fill_(nan)                                       # padding: never written by the kernel
+            mt.fill_(nan)
+            ops.explain_pairs(cs, dimp.struct(), int(model.config.batch_size), v[0], mt[1], mt[2], mt[0], v[2], v[1],
+                              dimp.work_counter)
+            o1 = dimp.order
+            oH = o1.view(b, k, 1).expand(b, k, H)
+            for dst, src in ((ex.score, v[0]), (ex.weight, v[1]), (ex.bias, v[2])):
+                dst[u0:u1].scatter_(1, o1, src.view(b, k))
+            for dst, src in ((ex.contrib, mt[0]), (ex.alpha, mt[1]), (ex.topic_attention, mt[2])):
+                dst[u0:u1].scatter_(1, oH, src.view(b, k, H))
+    return ex
